@@ -2,6 +2,7 @@
 """bench.py — mutated genome Gbp/s on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload c2|c1|c3|c4|c4d|c5|c1g]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over the whole synthetic genome: sample -> resolve -> link -> plan ->
 splice/emit FASTA image -> format VCF, all on the GPU (IT workloads: breakpoints -> exchange -> swap splice).
@@ -16,6 +17,8 @@ splice/emit FASTA image -> format VCF, all on the GPU (IT workloads: breakpoints
 `partition_invariant` (N > 1): every rank hashes its slices of the outputs on the device, rank 0 recomputes the
             whole genome alone with the same seed and compares — the N-GPU result IS the 1-GPU result.
 `--impl reference`: the reference's own CPU implementation on all host cores (one process per contig).
+`--dump-outputs DIR`: after the timed steps, the FASTA image and VCF body of the last one as float32 .npy files (see
+            dump_outputs), so that two builds can be compared output for output on the same seeded inputs.
 N > 1 (torchrun): contigs are partitioned over ranks (LPT by length, no data-path collective; for an IT pair that
 straddles ranks the splice kernel reads the partner's intervals in place from the peer GPU over NVLink, or —
 MS_IT_EXCHANGE=pull|nccl — they are copied / sent into a staging region); genomes with fewer contigs than ranks are cut at output
@@ -626,6 +629,33 @@ def measure(run: Run, steps, warmup, barrier, stream, local_rank, with_clocks=Fa
     return res
 
 
+DUMP_SEED = 2024
+DUMP_WINDOWS, DUMP_WINDOW = 1024, 4096        # per output: 4 MiB of bytes, 16 MiB as float32
+
+
+def dump_outputs(eng, out_dir: Path):
+    """Write what a caller of the last step receives: the FASTA image and the VCF body.  An output of at most
+    DUMP_WINDOWS * DUMP_WINDOW bytes is written whole, as one row; a larger one as DUMP_WINDOWS rows of DUMP_WINDOW
+    consecutive bytes at offsets drawn from its size with a fixed seed.  Files: fasta.npy / vcf.npy (byte values as
+    float32, one row per window), fasta_offsets.npy / vcf_offsets.npy (float64, where each row starts), sizes.npy
+    (float64: FASTA bytes, VCF bytes).  Under 33 MiB in all."""
+    from mutation_simulator_b200.engine import BUF_FASTA, BUF_VCF
+    out_dir.mkdir(parents=True, exist_ok=True)
+    sizes = []
+    for name, buf in (("fasta", BUF_FASTA), ("vcf", BUF_VCF)):
+        data = eng.download(buf)
+        sizes.append(len(data))
+        if len(data) <= DUMP_WINDOWS * DUMP_WINDOW:
+            offsets, rows = np.zeros(1, np.int64), data[None, :]
+        else:
+            rng = np.random.default_rng([DUMP_SEED, buf])
+            offsets = np.sort(rng.integers(0, len(data) - DUMP_WINDOW + 1, DUMP_WINDOWS))
+            rows = data[offsets[:, None] + np.arange(DUMP_WINDOW)]
+        np.save(out_dir / f"{name}.npy", rows.astype(np.float32))
+        np.save(out_dir / f"{name}_offsets.npy", offsets.astype(np.float64))
+    np.save(out_dir / "sizes.npy", np.array(sizes, np.float64))
+
+
 def roofline_of(run: Run, res):
     """k_splice: algorithmic bytes (SURVEY.md §8d: L + L' + ceil(L'/bpl) + 32 M + sum of TLI sources) / CUDA-event time
     of the stage, this rank's share; `emit` adds the VCF kernel (32 M read + line bytes written)."""
@@ -774,12 +804,18 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--no-invariance", action="store_true", help="skip the N-GPU == 1-GPU hash check")
     ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the FASTA image and VCF body of the last timed step into DIR as .npy files")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs is not None and (world > 1 or args.impl == "reference"):
+        ap.error("--dump-outputs needs the GPU implementation in a single process")
 
     if args.impl == "reference":
         reference_arm(args, wl, rank, world)
@@ -801,6 +837,8 @@ def main():
 
     run = Run(args.workload, rank, world, local_rank, stream)
     res = measure(run, args.steps, args.warmup, barrier, stream, local_rank, with_clocks=True)
+    if args.dump_outputs is not None:          # before anything below runs more steps on the same engine
+        dump_outputs(run.eng, args.dump_outputs)
     roofline = roofline_of(run, res)
     fasta_bytes, vcf_bytes = res["sizes"]
     invariant = None

@@ -1,8 +1,5 @@
 """SURVEY.md §8 f4: the GFF -> RMT helper and the annotation-derived RMTs it produces (overlapping blocked ranges)."""
 import re
-import subprocess
-import sys
-from pathlib import Path
 
 import numpy as np
 import pytest
@@ -10,9 +7,6 @@ import pytest
 from mutation_simulator_b200 import SimulationSettings, plan
 from mutation_simulator_b200.fasta import FastaRecord
 from mutation_simulator_b200.tools import gff_genes_2_rmt
-
-REF_RMTS = Path("/root/reference/data/Example RMT files")
-REF_SCRIPT = Path("/root/reference/data/scripts/gff_genes_2_rmt.py")
 
 GFF = """##gff-version 3
 chr2\tsrc\tgene\t500\t900\t.\t+\t.\tID=g1
@@ -46,12 +40,9 @@ def test_gff_helper_writes_what_the_reference_script_writes(tmp_path):
     (tmp_path / "a.gff3").write_text(GFF)
     assert gff_genes_2_rmt.main([str(tmp_path / "a.gff3"), "0.01"]) == 0
     got = (tmp_path / "a.rmt").read_text()
+    # what the reference's data/scripts/gff_genes_2_rmt.py writes for GFF
     assert got == ("std\nit None\nsn 0.01\n\nchr 1 #chr2\n500-900 None\n10-20 None\n"
                    "chr 2 #chr1\n100-400 None\n350-800 None\n360-370 None\n")
-    if REF_SCRIPT.exists():   # the unmodified reference script on the same input (build container only)
-        (tmp_path / "b.gff3").write_text(GFF)
-        subprocess.check_call([sys.executable, str(REF_SCRIPT), str(tmp_path / "b.gff3"), "0.01"])
-        assert (tmp_path / "b.rmt").read_text() == got
     assert gff_genes_2_rmt.main([str(tmp_path / "a.gff3")]) == 1
     assert gff_genes_2_rmt.main([str(tmp_path / "nope.gff3"), "0.1"]) == 1
     assert gff_genes_2_rmt.main([str(tmp_path / "a.gff3"), "x"]) == 1
@@ -73,10 +64,44 @@ def test_overlapping_blocked_ranges_are_planned_as_their_union(tmp_path):
         assert arr[i].k == int(((arr[i].stop - arr[i].start) + 1) * 0.01)
 
 
-@pytest.mark.skipif(not REF_RMTS.exists(), reason="reference data only exists in the build container")
-@pytest.mark.parametrize("name", ["Arabidopsis_thaliana", "Danio_rerio", "Drosophila_melanogaster", "Homo_sapiens", "Mus_musculus"])
-def test_shipped_example_rmts_parse_and_plan(name):
-    p = REF_RMTS / f"{name}.rmt"
+# name: (sequences, genes per sequence, sequence length, longest gene)
+ANNOTATIONS = {
+    "one_chromosome": (1, 3000, 120_000_000, 100_000),
+    "five_chromosomes": (5, 1000, 30_000_000, 100_000),
+    "twenty_five_chromosomes": (25, 200, 20_000_000, 100_000),
+    "dense_nested_genes": (3, 2500, 6_000_000, 5_000),
+    "many_scaffolds": (400, 5, 500_000, 50_000),
+}
+
+
+def annotation_gff(n_seq, genes, seq_len, longest, seed):
+    """A seeded genome annotation in GFF3: per sequence, genes of 200 bp to `longest` (log-uniform) at random places,
+    sorted by start as annotation files are, so that they overlap and nest like real genes; every gene carries an mRNA
+    and an exon, which the helper skips."""
+    rng = np.random.default_rng(seed)
+    out = ["##gff-version 3"]
+    for s in range(n_seq):
+        seqid = f"seq{s + 1}"
+        out.append(f"##sequence-region {seqid} 1 {seq_len}")
+        lens = np.exp(rng.uniform(np.log(200), np.log(longest), genes)).astype(np.int64)
+        starts = rng.integers(1, seq_len - lens + 1)
+        for g, i in enumerate(np.argsort(starts, kind="stable")):
+            a, b = int(starts[i]), int(starts[i] + lens[i] - 1)
+            strand = "+-"[g % 2]
+            out.append(f"{seqid}\tsynthetic\tgene\t{a}\t{b}\t.\t{strand}\t.\tID=g{s}_{g}")
+            out.append(f"{seqid}\tsynthetic\tmRNA\t{a}\t{b}\t.\t{strand}\t.\tID=t{s}_{g};Parent=g{s}_{g}")
+            out.append(f"{seqid}\tsynthetic\texon\t{a}\t{min(b, a + 150)}\t.\t{strand}\t.\tParent=t{s}_{g}")
+    return "\n".join(out) + "\n"
+
+
+@pytest.mark.parametrize("name", sorted(ANNOTATIONS))
+def test_annotation_rmts_parse_and_plan(name, tmp_path):
+    """RMTs the GFF helper makes from whole-genome annotations: thousands of overlapping and nested None ranges over
+    many sequences parse, and plan into sorted, in-bounds ranges that never touch a blocked interval."""
+    gff = tmp_path / f"{name}.gff3"
+    gff.write_text(annotation_gff(*ANNOTATIONS[name], seed=1))
+    assert gff_genes_2_rmt.main([str(gff), "0.01"]) == 0
+    p = gff.with_suffix(".rmt")
     ends, cur = {}, None
     for line in p.read_text().splitlines():
         m = re.match(r"chr (\d+)", line)
