@@ -196,7 +196,8 @@ int ms_apply_window(ms_ctx* ctx, int32_t part, int32_t n_parts, int64_t* window)
 int ms_mutate_streamed(ms_ctx* ctx, uint64_t seed, const uint8_t* bases, uint8_t* fasta, int64_t fasta_cap,
                        uint8_t* vcf, int64_t vcf_cap, int64_t* fasta_bytes, int64_t* vcf_bytes,
                        int64_t group_min_bases);
-/* which: 0 FASTA image, 1 VCF body, 2 records (ms_rec[]), 3 literal pool */
+/* which: 0 FASTA image, 1 VCF body, 2 records (ms_rec[]), 3 literal pool, 4 resident genome, 5 BGZF output of the
+ * last ms_bgzf_compress */
 int ms_download(ms_ctx* ctx, int which, void* dst, int64_t cap, int64_t* nbytes);
 int ms_device_ptr(ms_ctx* ctx, int which, void** dptr, int64_t* nbytes);
 /* Stream bytes [src_off, src_off+nbytes) of an output buffer into an open file at file_off: D2H through two pinned
@@ -231,6 +232,22 @@ int ms_sample_positions(ms_ctx* ctx, uint64_t seed, int32_t n, const uint32_t* g
  * geometry gives the same value.  bench.py uses it to check that the N-GPU outputs are the 1-GPU outputs without
  * moving them off the devices (SURVEY.md §4.5: results must not depend on the GPU count). */
 int ms_hash_ranges(ms_ctx* ctx, int which, int32_t n, const int64_t* start, const int64_t* end, uint64_t* out);
+
+/* ---- BGZF output ---------------------------------------------------------
+ * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body) into BGZF members on the device; the members,
+ * back to back in segment order, become buffer 5 (ms_download, ms_download_to_fd, ms_device_ptr, ms_hash_ranges).
+ * Segment s is bytes [src_off[s], src_off[s] + nbytes[s]) of the buffer, followed by one '\n' when add_nl[s] is 1
+ * (add_nl may be NULL), and starts at byte file_off[s] of the uncompressed file.  Members never span two segments
+ * and are cut at multiples of 16 KiB of the file, so a member is a pure function of the file's bytes and of where
+ * the segments begin: pass one segment per contig (ms_contig_layout) and several GPUs write the same file as one.
+ * Each member is a literal-only dynamic-Huffman deflate block, or a stored block when that is smaller (a member is
+ * at most its input + 31 bytes).  seg_zbytes[s] receives segment s's compressed size; the caller appends the 28-byte
+ * BGZF end-of-file member. */
+int ms_bgzf_compress(ms_ctx* ctx, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes,
+                     const int64_t* file_off, const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes);
+/* The same encoder on the host for small data (the VCF header): src[0..n) as members of 16 KiB each into dst.
+ * dst = NULL queries an upper bound of the size.  ctx may be NULL (no device is used). */
+int ms_bgzf_compress_host(ms_ctx* ctx, const uint8_t* src, int64_t n, uint8_t* dst, int64_t cap, int64_t* zbytes);
 
 /* ---- introspection ------------------------------------------------------ */
 int ms_get_stats(ms_ctx* ctx, ms_stats* out);

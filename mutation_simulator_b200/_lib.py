@@ -79,6 +79,8 @@ PROTOTYPES = {
     "ms_get_stats": (C.c_int, [_P, C.POINTER(MsStats)]),
     "ms_stage_name": (C.c_char_p, [C.c_int]),
     "ms_debug_candidates": (C.c_int, [_P, _I64, _P, _P, _P, _P, C.POINTER(_I64)]),
+    "ms_bgzf_compress": (C.c_int, [_P, C.c_int, _I32, _P, _P, _P, _P, _P, C.POINTER(_I64)]),
+    "ms_bgzf_compress_host": (C.c_int, [_P, _P, _I64, _P, _I64, C.POINTER(_I64)]),
 }
 
 _lib = None

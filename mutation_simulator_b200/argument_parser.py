@@ -1,7 +1,8 @@
 """Command line of ``mutation-simulator`` — flag for flag the reference's
-(argument_parser.py:31-240) plus two extensions that default to the reference's
+(argument_parser.py:31-240) plus three extensions that default to the reference's
 behaviour: ``--seed`` (reproducible runs; default: a fresh random seed, like the
-reference's unseeded RNGs) and ``--device`` (CUDA device index).
+reference's unseeded RNGs), ``--device`` (CUDA device index) and ``--bgzip``
+(BGZF-compressed FASTA and VCF output, encoded on the GPU).
 
 The option table below drives argparse; the derived output names follow
 argument_parser.py:14-28."""
@@ -32,6 +33,10 @@ def add_outfile_names(args: Namespace) -> Namespace:
     args.outfastait = args.outfasta.with_stem(args.outfasta.stem + "_it")
     args.outvcf = args.outfasta.with_suffix(".vcf")
     args.outbedpe = args.outfastait.with_suffix(".bedpe")
+    if getattr(args, "bgzip", False):      # after the derivation: *_it and .bedpe keep their names
+        for k in ("outfasta", "outfastait", "outvcf"):
+            p = getattr(args, k)
+            setattr(args, k, p.with_name(p.name + ".gz"))
     return args
 
 
@@ -50,6 +55,8 @@ def build_parser() -> ArgumentParser:
     p.add_argument("--seed", type=int, default=None,
                    help="[extension] seed of the counter-based RNG; default: a fresh random seed per run")
     p.add_argument("--device", type=int, default=0, help="[extension] CUDA device index. Default = 0")
+    p.add_argument("--bgzip", action="store_true", default=False,
+                   help="[extension] write the FASTA and VCF outputs BGZF-compressed (names get .gz); the BEDPE stays plain")
 
     sub = p.add_subparsers(dest="mode", help="Generate mutations or interchromosomal translocations via RMT or arguments")
     sub.required = True

@@ -3,10 +3,12 @@
 #include <errno.h>
 #include <string.h>
 #include <unistd.h>
+#include <algorithm>
 #include <future>
 #include <sys/mman.h>
 #include <sys/stat.h>
 #include <sys/statvfs.h>
+#include "ms_bgzf_core.h"
 #include "ms_common.cuh"
 
 using namespace ms;
@@ -78,7 +80,8 @@ int ms_destroy(ms_ctx* c) {
                       &c->bucket_cnt, &c->bucket_off, &c->cand_type, &c->cand_len, &c->cand_reach, &c->cand_pm, &c->cand_accept,
                       &c->acc_idx, &c->tl_list, &c->tli_list, &c->link, &c->keep, &c->contig_tl, &c->scan_tmp, &c->scan_tmp2,
                       &c->svec, &c->vvec, &c->lvec, &c->tmp_contigs, &c->recs, &c->lit, &c->scan_mid, &c->nvec, &c->sv_stream, &c->snp_stream, &c->piece_lo, &c->piece_desc, &c->fasta, &c->vcf,
-                      &c->vcf_off, &c->totals, &c->bucket_range, &c->vend, &c->fa_index};
+                      &c->vcf_off, &c->totals, &c->bucket_range, &c->vend, &c->fa_index, &c->bgzf, &c->bgzf_blocks,
+                      &c->bgzf_slots, &c->bgzf_zsize};
     for (DevBuf* b : bufs) b->release();
     for (cudaStream_t* s : {&c->s_up, &c->s_down, &c->s_vcf})
         if (*s) { cudaStreamSynchronize(*s); cudaStreamDestroy(*s); }
@@ -444,6 +447,7 @@ static int which_buffer(ms_ctx* c, int which, void** p, int64_t* n) {
                 *p = c->recs.p; *n = c->n_recs * (int64_t)sizeof(Rec); return MS_OK;
         case 3: *p = c->lit.p; *n = c->lit_bytes; return MS_OK;
         case 4: *p = c->genome.p; *n = c->total_bases; return MS_OK;
+        case 5: *p = c->bgzf.p; *n = c->bgzf_bytes; return MS_OK;
         default: MS_FAIL(c, MS_ERR_ARG, "unknown buffer id %d", which);
     }
 }
@@ -607,6 +611,36 @@ int ms_hash_ranges(ms_ctx* c, int which, int32_t n, const int64_t* start, const 
             MS_FAIL(c, MS_ERR_ARG, "ms_hash_ranges: range %d is outside the buffer or not in ascending order", i);
     MS_CUDA(c, cudaSetDevice(c->device));
     return hash_ranges(c, static_cast<const uint8_t*>(p), n, start, end, out);
+}
+
+int ms_bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
+                     const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes) {
+    if (!c || (which != 0 && which != 1) || n_seg < 0 || !total_zbytes ||
+        (n_seg > 0 && (!src_off || !nbytes || !file_off || !seg_zbytes)))
+        return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return bgzf_compress(c, which, n_seg, src_off, nbytes, file_off, add_nl, seg_zbytes, total_zbytes);
+}
+
+int ms_bgzf_compress_host(ms_ctx* c, const uint8_t* src, int64_t n, uint8_t* dst, int64_t cap, int64_t* zbytes) {
+    if (n < 0 || (n > 0 && !src) || !zbytes) return MS_ERR_ARG;
+    const int64_t need = ((n + bgzf::CELL - 1) / bgzf::CELL) * bgzf::MAX_MEMBER;
+    *zbytes = 0;
+    if (!dst) { *zbytes = need; return MS_OK; }     // size query: an upper bound
+    std::vector<uint8_t> member(bgzf::MAX_MEMBER);
+    int64_t o = 0;
+    for (int64_t i = 0; i < n; i += bgzf::CELL) {
+        const int m = (int)std::min<int64_t>(bgzf::CELL, n - i);
+        const int z = bgzf::encode_member(src + i, m, member.data());
+        if (o + z > cap) {
+            if (c) MS_FAIL(c, MS_ERR_ARG, "ms_bgzf_compress_host: output buffer too small");
+            return MS_ERR_ARG;
+        }
+        memcpy(dst + o, member.data(), (size_t)z);
+        o += z;
+    }
+    *zbytes = o;
+    return MS_OK;
 }
 
 int ms_get_stats(ms_ctx* c, ms_stats* out) {

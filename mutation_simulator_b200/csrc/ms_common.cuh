@@ -130,6 +130,10 @@ struct ms_ctx {
     ms::DevBuf vend;                 // VCF bytes up to the end of each contig group
     int64_t* h_vend = nullptr;       // pinned copy
     size_t h_vend_cap = 0;
+
+    // BGZF output of the last ms_bgzf_compress (buffer 5), its block table and per-member scratch
+    ms::DevBuf bgzf, bgzf_blocks, bgzf_slots, bgzf_zsize;
+    int64_t bgzf_bytes = 0;
 };
 
 #define MS_CUDA(ctx, call)                                                                        \
@@ -177,4 +181,6 @@ int mutate_streamed(ms_ctx* c, uint64_t seed, const uint8_t* h_bases, uint8_t* h
 int count_types(ms_ctx* c);
 int fill_record_out(ms_ctx* c);
 int hash_ranges(ms_ctx* c, const uint8_t* buf, int32_t n, const int64_t* start, const int64_t* end, uint64_t* out);
+int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
+                  const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes);
 }  // namespace ms

@@ -221,9 +221,13 @@ def _create(path, prefix: bytes, total: int):
         raise OutputCreateError(err)
 
 
-def write_window(path, engine, which, lo: int, hi: int, total: int, prefix: bytes = b""):
+def write_window(path, engine, which, lo: int, hi: int, total: int, prefix: bytes = b"", bgzip: bool = False):
     """Tile-sharded runs: this rank produced bytes [lo, hi) of device buffer `which`, whose layout is the same on every
-    rank; all ranks stream their ranges into one file of `total` bytes after `prefix`."""
+    rank; all ranks stream their ranges into one file of `total` bytes after `prefix`.  bgzip: each rank compresses
+    the contig slices of its window (the FASTA windows start on 16 KiB cells, so the members are the 1-GPU run's),
+    the compressed sizes are gathered in rank order, and the last rank appends the EOF member."""
+    if bgzip:
+        return _write_window_bgzf(path, engine, which, lo, hi, prefix)
     _create(path, prefix, len(prefix) + int(total))
     if hi > lo:
         fd = os.open(path, os.O_RDWR)
@@ -234,10 +238,14 @@ def write_window(path, engine, which, lo: int, hi: int, total: int, prefix: byte
     barrier()
 
 
-def write_slices_partitioned(path, engine, which, my_ids, slice_off, n_contigs, prefix: bytes = b""):
+def write_slices_partitioned(path, engine, which, my_ids, slice_off, n_contigs, prefix: bytes = b"", bgzip: bool = False):
     """Contig i of this rank owns bytes [slice_off[i], slice_off[i+1]) of device buffer `which`; all ranks stream
     their slices into one file, contigs in global order, without passing through Python."""
     sizes = [int(slice_off[i + 1] - slice_off[i]) for i in range(len(my_ids))]
+    if bgzip:
+        off = _global_offsets(my_ids, sizes, n_contigs, 0)
+        return _write_contigs_bgzf(path, engine, which, my_ids, [int(slice_off[i]) for i in range(len(my_ids))], sizes,
+                                   off, [0] * len(my_ids), n_contigs, prefix)
     off = _global_offsets(my_ids, sizes, n_contigs, len(prefix))
     _create(path, prefix, off[-1])
     fd = os.open(path, os.O_RDWR)
@@ -257,7 +265,7 @@ def write_slices_partitioned(path, engine, which, my_ids, slice_off, n_contigs, 
     barrier()
 
 
-def write_fasta_partitioned(path, engine, my_ids, n_contigs_global):
+def write_fasta_partitioned(path, engine, my_ids, n_contigs_global, bgzip: bool = False):
     """FASTA image slices with the separator fixed up for the global file order (a '\\n' follows a partial last
     line unless the contig is the last one of the whole file).  Returns the per-contig VCF offsets of the layout."""
     if len(my_ids) == 0:      # more ranks than contigs: this rank only takes part in the collectives
@@ -267,6 +275,10 @@ def write_fasta_partitioned(path, engine, my_ids, n_contigs_global):
     body = [int(fo[i + 1] - fo[i]) - int(sep[i]) for i in range(len(my_ids))]
     extra = [1 if (partial[i] and g != n_contigs_global - 1) else 0 for i, g in enumerate(my_ids)]
     off = _global_offsets(my_ids, [b + e for b, e in zip(body, extra)], n_contigs_global, 0)
+    if bgzip:
+        _write_contigs_bgzf(path, engine, 0, my_ids, [int(fo[i]) for i in range(len(my_ids))], body, off, extra,
+                            n_contigs_global, b"")
+        return vo
     _create(path, b"", off[-1])
     from .engine import BUF_FASTA
     fd = os.open(path, os.O_RDWR)
@@ -280,3 +292,60 @@ def write_fasta_partitioned(path, engine, my_ids, n_contigs_global):
         os.close(fd)
     barrier()
     return vo
+
+
+def _write_contigs_bgzf(path, engine, which, my_ids, src, nbytes, file_off, add_nl, n_contigs, prefix: bytes):
+    """Contig-sharded BGZF: contig i of this rank is nbytes[i] bytes of buffer `which` at src[i] (+ '\\n' if
+    add_nl[i]) and starts at file_off[global id] of the uncompressed file (the first all-gather); each rank compresses
+    its contigs, a second all-gather of the compressed sizes places them, rank 0 writes the compressed prefix and the
+    owner of the last contig the EOF member."""
+    from .bgzf import EOF, compress_host
+    from .engine import BUF_BGZF
+    zhead = compress_host(prefix)
+    if len(my_ids):
+        zseg, _ = engine.bgzf_compress(which, src, nbytes, [int(file_off[g]) for g in my_ids], add_nl)
+    else:
+        zseg = np.zeros(0, np.int64)
+    zoff = _global_offsets(my_ids, [int(z) for z in zseg], n_contigs, len(zhead))
+    _create(path, zhead, int(zoff[-1]) + len(EOF))
+    fd = os.open(path, os.O_RDWR)
+    try:
+        local = np.concatenate(([0], np.cumsum(zseg))).astype(np.int64)
+        i = 0
+        while i < len(my_ids):          # consecutive contigs are consecutive in buffer 5 and in the file
+            j = i
+            while j + 1 < len(my_ids) and my_ids[j + 1] == my_ids[j] + 1:
+                j += 1
+            n = int(local[j + 1] - local[i])
+            if n:
+                engine.download_to_fd(BUF_BGZF, fd, int(zoff[my_ids[i]]), int(local[i]), n)
+            i = j + 1
+        if n_contigs - 1 in my_ids:
+            os.pwrite(fd, EOF, int(zoff[-1]))
+    finally:
+        os.close(fd)
+    barrier()
+
+
+def _write_window_bgzf(path, engine, which, lo: int, hi: int, prefix: bytes):
+    from .bgzf import EOF, compress_host, window_segments
+    from .engine import BUF_BGZF
+    zhead = compress_host(prefix)
+    tot = 0
+    if hi > lo:
+        src, n = window_segments(engine, which, int(lo), int(hi))
+        _, tot = engine.bgzf_compress(which, src, n, src)
+    sizes = all_gather_object(int(tot))
+    rank = rank_world()[0]
+    at = len(zhead) + sum(sizes[:rank])
+    end = len(zhead) + sum(sizes)
+    _create(path, zhead, end + len(EOF))
+    fd = os.open(path, os.O_RDWR)
+    try:
+        if tot:
+            engine.download_to_fd(BUF_BGZF, fd, at, 0, tot)
+        if rank == len(sizes) - 1:
+            os.pwrite(fd, EOF, end)
+    finally:
+        os.close(fd)
+    barrier()

@@ -14,11 +14,26 @@ from . import _lib
 from ._lib import MsRange, MsStats, MutSimError
 from .records import REC_DTYPE
 
-BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME = range(5)
+BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF = range(6)
 
 
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def bgzf_compress_host(data: bytes) -> bytes:
+    """BGZF members (16 KiB of input each) of small host data with the device's encoder (ms_bgzf_compress_host);
+    needs the library, not a GPU."""
+    lib = _lib.load()
+    src = np.frombuffer(bytes(data), dtype=np.uint8)
+    cap = C.c_int64()
+    rc = lib.ms_bgzf_compress_host(None, _ptr(src), src.size, None, 0, C.byref(cap))
+    out = np.empty(max(cap.value, 1), dtype=np.uint8)
+    n = C.c_int64()
+    rc = rc or lib.ms_bgzf_compress_host(None, _ptr(src), src.size, _ptr(out), out.size, C.byref(n))
+    if rc:
+        raise MutSimError(rc, "ms_bgzf_compress_host failed")
+    return out[:n.value].tobytes()
 
 
 def _blob(items: Sequence[bytes]):
@@ -279,6 +294,18 @@ class Engine:
             nbytes = self.size_of(which) - src_off
         self._check(self._lib.ms_download_to_fd(self._h, which, int(src_off), int(nbytes), int(fd), int(file_off)))
         return int(nbytes)
+
+    def bgzf_compress(self, which: int, src_off, nbytes, file_off, add_nl=None):
+        """BGZF members of segments of the FASTA image (which=0) or the VCF body (which=1), cut on 16 KiB cells of
+        the uncompressed file (ms_bgzf_compress); they become buffer BUF_BGZF.  Returns (compressed bytes of each
+        segment, total)."""
+        src_off, nbytes, file_off = (np.ascontiguousarray(a, dtype=np.int64) for a in (src_off, nbytes, file_off))
+        nl = None if add_nl is None else np.ascontiguousarray(add_nl, dtype=np.uint8)
+        seg = np.zeros(len(src_off), dtype=np.int64)
+        tot = C.c_int64()
+        self._check(self._lib.ms_bgzf_compress(self._h, int(which), len(src_off), _ptr(src_off), _ptr(nbytes), _ptr(file_off),
+                                               _ptr(nl), _ptr(seg), C.byref(tot)))
+        return seg, tot.value
 
     def fasta(self) -> bytes:
         return self.download(BUF_FASTA).tobytes()

@@ -16,6 +16,8 @@ from pathlib import Path
 
 import numpy as np
 
+from .bgzf import inflate_if_compressed
+
 _UPPER = np.arange(256, dtype=np.uint8)
 _UPPER[ord("a"):ord("z") + 1] -= 32
 
@@ -100,7 +102,9 @@ class Fasta:
 
     def __init__(self, filename, one_based_attributes=False, as_raw=True, sequence_always_upper=True,
                  read_ahead=None, build_index=True, device=None, **_):
-        """device: CUDA device index — the file is then ingested on that GPU (ms_fasta_ingest_fd: raw bytes to HBM,
+        """A BGZF-compressed file (``--bgzip`` output, or ``bgzip``) is inflated on the host and parsed there; the .fai
+        then holds offsets into the uncompressed text, as ``samtools faidx`` writes them.
+        device: CUDA device index — the file is then ingested on that GPU (ms_fasta_ingest_fd: raw bytes to HBM,
         records / line layout / stripping / upper-casing there) and `self.engine` holds the resident genome for the
         Mutator / ITMutator that follows; host views of the bases are fetched from the device on demand.  Files that
         are not regularly wrapped, and device=None, go through the host parsers."""
@@ -110,7 +114,10 @@ class Fasta:
         self._genome = None
         self.engine = None
         try:
-            if device is not None and self._ingest_device(int(device)):
+            inflated = inflate_if_compressed(self.filename)     # BGZF input: inflated on the host, then the host parser
+            if inflated is not None:
+                self._parse(np.frombuffer(inflated, dtype=np.uint8), sequence_always_upper)
+            elif device is not None and self._ingest_device(int(device)):
                 pass
             elif not self._parse_regular():
                 self._parse(np.fromfile(self.filename, dtype=np.uint8), sequence_always_upper)

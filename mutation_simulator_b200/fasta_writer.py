@@ -10,7 +10,9 @@ class FastaWriterError(Exception):
 
 
 class FastaWriter:
-    def __init__(self, fname):
+    def __init__(self, fname, bgzip: bool = False):
+        """bgzip: write_from_engine writes BGZF (the per-base API below always writes plain text)."""
+        self._bgzip = bgzip
         try:
             self._f = open(fname, "w+b")   # read-write: libmutsim_b200 maps the file for its parallel writers
         except OSError as e:
@@ -31,6 +33,9 @@ class FastaWriter:
 
     def write_from_engine(self, engine, which: int):
         """Stream a device buffer straight into the file (pinned double buffering inside libmutsim_b200)."""
+        if self._bgzip:
+            from .bgzf import write_from_engine
+            return write_from_engine(self._f, engine, which)
         self._f.flush()
         off = self._f.tell()
         n = engine.download_to_fd(which, self._f.fileno(), off)

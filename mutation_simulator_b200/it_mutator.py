@@ -48,7 +48,7 @@ class ITMutator:
         self._args, self._fasta, self._sim = args, fasta, sim
         self._rank, self._world = D.init()
         if self._world == 1:
-            self._fasta_writer = FastaWriter(args.outfastait)
+            self._fasta_writer = FastaWriter(args.outfastait, getattr(args, "bgzip", False))
             self._bedpe_writer = BedpeWriter(args.outbedpe)
         else:
             self._fasta_writer = self._bedpe_writer = None
@@ -180,7 +180,7 @@ class ITMutator:
         bps = self.breakpoints = self._generate_all_breakpoints(eng)
         eng.load_records(self._records(bps))
         w = eng.apply_window(rank, world)
-        D.write_window(self._args.outfastait, eng, BUF_FASTA, *w["fasta"], w["fasta_bytes"])
+        D.write_window(self._args.outfastait, eng, BUF_FASTA, *w["fasta"], w["fasta_bytes"], bgzip=getattr(self._args, "bgzip", False))
         bed = b""
         if rank == 0:
             for chrom in self._sim.chromosomes:
@@ -302,7 +302,7 @@ class ITMutator:
     def write_partitioned(self):
         fasta, my_ids, bps = self._fasta, self._my_ids, self.breakpoints
         n_contigs = len(fasta.names)
-        D.write_fasta_partitioned(self._args.outfastait, self._engine, my_ids, n_contigs)
+        D.write_fasta_partitioned(self._args.outfastait, self._engine, my_ids, n_contigs, bgzip=getattr(self._args, "bgzip", False))
         bed = []
         for g in my_ids:
             if g in bps:

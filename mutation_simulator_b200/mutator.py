@@ -40,8 +40,9 @@ class Mutator:
         if self._world > 1:      # one process per GPU: files are assembled by write_partitioned()
             self._fasta_writer = self._vcf_writer = None
             return
-        self._fasta_writer = FastaWriter(args.outfasta)
-        self._vcf_writer = VcfWriter(args.outvcf)
+        bgzip = getattr(args, "bgzip", False)
+        self._fasta_writer = FastaWriter(args.outfasta, bgzip)
+        self._vcf_writer = VcfWriter(args.outvcf, bgzip)
         self._vcf_writer.write_header(args.infile.name, fasta, sim.assembly_name, sim.species_name, sim.sample_name)
 
     def load_vcf(self, text):
@@ -120,18 +121,19 @@ class Mutator:
             from .vcf_writer import VcfWriterError, header_text
             head = header_text(args.infile.name, [(fasta[k].name, len(fasta[k])) for k in fasta.keys()], sim.assembly_name,
                                sim.species_name, sim.sample_name).encode("latin-1")
+            bgzip = getattr(args, "bgzip", False)
             try:
                 if tiles:
-                    D.write_window(args.outfasta, eng, BUF_FASTA, *window["fasta"], window["fasta_bytes"])
+                    D.write_window(args.outfasta, eng, BUF_FASTA, *window["fasta"], window["fasta_bytes"], bgzip=bgzip)
                 else:
-                    vcf_off = D.write_fasta_partitioned(args.outfasta, eng, my_ids, n_contigs)
+                    vcf_off = D.write_fasta_partitioned(args.outfasta, eng, my_ids, n_contigs, bgzip=bgzip)
             except D.OutputCreateError as e:
                 raise FastaWriterError(f"Cannot write to Fasta file {args.outfasta} {e}")
             try:
                 if tiles:
-                    D.write_window(args.outvcf, eng, BUF_VCF, *window["vcf"], window["vcf_bytes"], prefix=head)
+                    D.write_window(args.outvcf, eng, BUF_VCF, *window["vcf"], window["vcf_bytes"], prefix=head, bgzip=bgzip)
                 else:
-                    D.write_slices_partitioned(args.outvcf, eng, BUF_VCF, my_ids, vcf_off, n_contigs, prefix=head)
+                    D.write_slices_partitioned(args.outvcf, eng, BUF_VCF, my_ids, vcf_off, n_contigs, prefix=head, bgzip=bgzip)
             except D.OutputCreateError as e:
                 raise VcfWriterError(f"Cannot write to VCF file {args.outvcf} {e}")
         lap("download+write")

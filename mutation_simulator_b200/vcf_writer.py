@@ -46,7 +46,9 @@ def header_text(input_fasta, contigs, assembly_name, species_name, sample_name, 
 
 
 class VcfWriter:
-    def __init__(self, fname):
+    def __init__(self, fname, bgzip: bool = False):
+        """bgzip: the header and write_from_engine's body are written as BGZF members (write / write_body stay plain)."""
+        self._bgzip = bgzip
         try:
             self._f = open(fname, "w+b")   # read-write: libmutsim_b200 maps the file for its parallel writers
         except OSError as e:
@@ -61,13 +63,20 @@ class VcfWriter:
 
     def write_header(self, input_fasta, fasta, assembly_name, species_name, sample_name):
         names = fasta.keys()
-        self._f.write(header_text(input_fasta, [(fasta[n].name, len(fasta[n])) for n in names], assembly_name, species_name,
-                                  sample_name).encode("latin-1"))
+        head = header_text(input_fasta, [(fasta[n].name, len(fasta[n])) for n in names], assembly_name, species_name,
+                           sample_name).encode("latin-1")
+        if self._bgzip:
+            from .bgzf import compress_host
+            head = compress_host(head)
+        self._f.write(head)
 
     def write_body(self, body):
         self._f.write(memoryview(body))
 
     def write_from_engine(self, engine, which: int):
+        if self._bgzip:
+            from .bgzf import write_from_engine
+            return write_from_engine(self._f, engine, which)
         self._f.flush()
         off = self._f.tell()
         n = engine.download_to_fd(which, self._f.fileno(), off)
