@@ -170,6 +170,18 @@ int ms_sample(ms_ctx* ctx, uint64_t seed);
  * Loads an explicit mutation table (what Mutator.__mutate_sequence receives as
  * `muts`, mutator.py:318) as splice descriptors sorted by (contig, pos). */
 int ms_load_records(ms_ctx* ctx, const ms_rec* recs, int64_t n_recs, const uint8_t* lit, int64_t lit_bytes);
+/* Parse VCF text (header lines skipped) into the context's record table and literal pool: what records_from_vcf
+ * (mutation_simulator_b200/records.py:119-191) + ms_load_records do, parsed on the device, for the regular shape of
+ * the lines VcfWriter.write emits (the reference's vcf_writer.py:118-126, and this package's VCF body): lines end in
+ * '\n' (no '\r' or other line breaks), >= 8 tab-separated fields, CHROM one of the resident contigs' names (lines of
+ * other contigs are dropped when skip_unknown is 1), POS ASCII digits, INFO '.' or exactly
+ * SVTYPE=<type>;END=<digits>;SVLEN=<digits>, every contig's lines in one block with increasing POS (blocks in any
+ * contig order), every record inside its contig.  The text is copied to the device in chunks.
+ * *regular = 0: nothing was loaded (the context is unchanged) and the caller must use the host parser.  *regular = 1:
+ * the table is byte-identical to records_from_vcf's, with literal offsets in file order; the checks of
+ * ms_load_records ran with its error codes, and *n_recs holds the number of records. */
+int ms_load_vcf(ms_ctx* ctx, const uint8_t* text, int64_t nbytes, int32_t skip_unknown,
+                int32_t* regular, int64_t* n_recs);
 
 /* ---- apply -------------------------------------------------------------
  * Replaces Mutator.__mutate_sequence (mutator.py:318-426) with FastaWriter

@@ -69,6 +69,7 @@ PROTOTYPES = {
     "ms_set_ranges": (C.c_int, [_P, _P, _I32, _P, _I32, C.c_double]),
     "ms_sample": (C.c_int, [_P, _U64]),
     "ms_load_records": (C.c_int, [_P, _P, _I64, _P, _I64]),
+    "ms_load_vcf": (C.c_int, [_P, _P, _I64, _I32, C.POINTER(_I32), C.POINTER(_I64)]),
     "ms_apply": (C.c_int, [_P, C.POINTER(_I64), C.POINTER(_I64)]),
     "ms_apply_window": (C.c_int, [_P, _I32, _I32, _P]),
     "ms_download": (C.c_int, [_P, C.c_int, _P, _I64, C.POINTER(_I64)]),

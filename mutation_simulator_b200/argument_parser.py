@@ -2,7 +2,8 @@
 (argument_parser.py:31-240) plus three extensions that default to the reference's
 behaviour: ``--seed`` (reproducible runs; default: a fresh random seed, like the
 reference's unseeded RNGs), ``--device`` (CUDA device index) and ``--bgzip``
-(BGZF-compressed FASTA and VCF output, encoded on the GPU).
+(BGZF-compressed FASTA and VCF output, encoded on the GPU), and the ``vcf`` mode
+(replay a VCF the reference or this package wrote onto the same FASTA).
 
 The option table below drives argparse; the derived output names follow
 argument_parser.py:14-28."""
@@ -79,6 +80,9 @@ def build_parser() -> ArgumentParser:
     it.add_argument("interchromosomalrate", type=float, help="Rate of interchromosomal translocations")
     rmt = sub.add_parser("rmt", help="Use random mutation table instead of arguments")
     rmt.add_argument("rmtfile", type=Path, help="Path to the RMT file")
+    vcf = sub.add_parser("vcf", help="[extension] Apply the mutations of a VCF written by Mutation-Simulator to the Fasta "
+                                     "(writes the *_ms.fa it describes and re-emits the VCF)")
+    vcf.add_argument("vcffile", type=Path, help="Path to the VCF file (plain, gzip or BGZF)")
     return p
 
 

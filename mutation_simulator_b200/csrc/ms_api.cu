@@ -15,6 +15,27 @@ using namespace ms;
 
 static thread_local std::string g_create_error;
 
+namespace ms {
+// The error ms_load_records reports for record i failing check `fault` (rec_fault).
+int record_fault(ms_ctx* c, int fault, int64_t i) {
+    switch (fault) {
+        case RF_CONTIG: MS_FAIL(c, MS_ERR_ARG, "record %lld: contig out of range", (long long)i);
+        case RF_ORDER: MS_FAIL(c, MS_ERR_OVERLAP, "record %lld: records must be sorted by (contig, pos) with distinct positions", (long long)i);
+        case RF_LIT: MS_FAIL(c, MS_ERR_ARG, "record %lld: literal range outside the pool", (long long)i);
+        default: MS_FAIL(c, MS_ERR_ARG, "record %lld: source range outside the genome", (long long)i);
+    }
+}
+
+// The record table and literal pool of c are now a loaded table (ms_load_records, ms_load_vcf).
+void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes) {
+    c->n_recs = n_recs;
+    c->lit_bytes = lit_bytes;
+    c->counts_valid = false;
+    c->sizes_valid = false;
+    c->rec_out_valid = true;
+}
+}  // namespace ms
+
 static const char* STAGE_NAMES[ST_COUNT] = {"upload", "sample_positions", "sample_type_len", "sample_resolve",
                                             "sample_link", "sample_finalize", "plan_scan_layout", "block_index",
                                             "splice_emit_fasta", "vcf_format", "download"};
@@ -81,7 +102,8 @@ int ms_destroy(ms_ctx* c) {
                       &c->acc_idx, &c->tl_list, &c->tli_list, &c->link, &c->keep, &c->contig_tl, &c->scan_tmp, &c->scan_tmp2,
                       &c->svec, &c->vvec, &c->lvec, &c->tmp_contigs, &c->recs, &c->lit, &c->scan_mid, &c->nvec, &c->sv_stream, &c->snp_stream, &c->piece_lo, &c->piece_desc, &c->fasta, &c->vcf,
                       &c->vcf_off, &c->totals, &c->bucket_range, &c->vend, &c->fa_index, &c->bgzf, &c->bgzf_blocks,
-                      &c->bgzf_slots, &c->bgzf_zsize};
+                      &c->bgzf_slots, &c->bgzf_zsize, &c->vp_text, &c->vp_lines, &c->vp_lrec, &c->vp_krec,
+                      &c->vp_lit, &c->vp_names, &c->vp_contig};
     for (DevBuf* b : bufs) b->release();
     for (cudaStream_t* s : {&c->s_up, &c->s_down, &c->s_vcf})
         if (*s) { cudaStreamSynchronize(*s); cudaStreamDestroy(*s); }
@@ -397,16 +419,11 @@ int ms_load_records(ms_ctx* c, const ms_rec* recs, int64_t n_recs, const uint8_t
     if (!c || n_recs < 0 || lit_bytes < 0 || (n_recs > 0 && !recs)) return MS_ERR_ARG;
     if (c->n_contigs <= 0) MS_FAIL(c, MS_ERR_STATE, "ms_load_records: upload a genome first");
     static_assert(sizeof(ms_rec) == sizeof(Rec), "ms_rec layout");
+    const Rec* r = reinterpret_cast<const Rec*>(recs);
     for (int64_t i = 0; i < n_recs; ++i) {
-        if (recs[i].contig >= (uint32_t)c->n_contigs) MS_FAIL(c, MS_ERR_ARG, "record %lld: contig out of range", (long long)i);
-        if (i && (recs[i].contig < recs[i - 1].contig || (recs[i].contig == recs[i - 1].contig && recs[i].pos <= recs[i - 1].pos)))
-            MS_FAIL(c, MS_ERR_OVERLAP, "record %lld: records must be sorted by (contig, pos) with distinct positions", (long long)i);
-        if (recs[i].kind == K_LIT && (recs[i].src < 0 || recs[i].src + recs[i].prod > lit_bytes))
-            MS_FAIL(c, MS_ERR_ARG, "record %lld: literal range outside the pool", (long long)i);
-        if ((recs[i].kind == K_RAW || recs[i].kind == K_CONV || recs[i].kind == K_RC) &&
-            (recs[i].src < 0 || recs[i].src + recs[i].prod > c->total_bases + 64 + c->foreign_cap) &&
-            !(recs[i].kind == K_RAW && source_in_peer_window(c, recs[i].src, recs[i].prod)))
-            MS_FAIL(c, MS_ERR_ARG, "record %lld: source range outside the genome", (long long)i);
+        int f = rec_fault(r, i, c->n_contigs, lit_bytes, c->total_bases + 64 + c->foreign_cap);
+        if (f == RF_SRC && r[i].kind == K_RAW && source_in_peer_window(c, r[i].src, r[i].prod)) f = RF_OK;
+        if (f) return record_fault(c, f, i);
     }
     MS_CUDA(c, cudaSetDevice(c->device));
     MS_CUDA(c, c->recs.ensure((size_t)(n_recs + 1) * sizeof(Rec)));
@@ -414,12 +431,16 @@ int ms_load_records(ms_ctx* c, const ms_rec* recs, int64_t n_recs, const uint8_t
     if (n_recs) MS_CUDA(c, cudaMemcpyAsync(c->recs.p, recs, (size_t)n_recs * sizeof(Rec), cudaMemcpyHostToDevice, c->stream));
     if (lit_bytes) MS_CUDA(c, cudaMemcpyAsync(c->lit.p, lit, (size_t)lit_bytes, cudaMemcpyHostToDevice, c->stream));
     MS_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->n_recs = n_recs;
-    c->lit_bytes = lit_bytes;
-    c->counts_valid = false;
-    c->sizes_valid = false;
-    c->rec_out_valid = true;
+    records_loaded(c, n_recs, lit_bytes);
     return MS_OK;
+}
+
+int ms_load_vcf(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t* regular, int64_t* n_recs) {
+    if (!c || nbytes < 0 || (nbytes > 0 && !text) || !regular || !n_recs) return MS_ERR_ARG;
+    *regular = 0; *n_recs = 0;
+    if (c->n_contigs <= 0) MS_FAIL(c, MS_ERR_STATE, "ms_load_vcf: upload a genome first");
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return vcf_load(c, text, nbytes, skip_unknown, regular, n_recs);
 }
 
 // ---- apply ----------------------------------------------------------------------------

@@ -134,6 +134,10 @@ struct ms_ctx {
     // BGZF output of the last ms_bgzf_compress (buffer 5), its block table and per-member scratch
     ms::DevBuf bgzf, bgzf_blocks, bgzf_slots, bgzf_zsize;
     int64_t bgzf_bytes = 0;
+
+    // ms_load_vcf: text, line starts, per-line records (then the new table), compacted records, the new literal pool,
+    // the CHROM hash table, scalars and per-contig block bounds
+    ms::DevBuf vp_text, vp_lines, vp_lrec, vp_krec, vp_lit, vp_names, vp_contig;
 };
 
 #define MS_CUDA(ctx, call)                                                                        \
@@ -181,6 +185,9 @@ int mutate_streamed(ms_ctx* c, uint64_t seed, const uint8_t* h_bases, uint8_t* h
 int count_types(ms_ctx* c);
 int fill_record_out(ms_ctx* c);
 int hash_ranges(ms_ctx* c, const uint8_t* buf, int32_t n, const int64_t* start, const int64_t* end, uint64_t* out);
+int vcf_load(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t* regular, int64_t* n_recs);
+int record_fault(ms_ctx* c, int fault, int64_t i);
+void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes);
 int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                   const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes);
 }  // namespace ms

@@ -64,6 +64,18 @@ struct Contig {
     uint32_t pad;
 };
 
+// What ms_load_records requires of record i of a table r (checked in this order): RF_OK or the first check it fails.
+// src_end = end of the genome buffer (resident bases, pad and staging region) that K_RAW / K_CONV / K_RC sources index.
+enum RecFault : int { RF_OK = 0, RF_CONTIG = 1, RF_ORDER = 2, RF_LIT = 3, RF_SRC = 4 };
+MS_HD int rec_fault(const Rec* r, int64_t i, int32_t n_contigs, int64_t lit_bytes, int64_t src_end) {
+    const Rec& x = r[i];
+    if (x.contig >= (uint32_t)n_contigs) return RF_CONTIG;
+    if (i && (x.contig < r[i - 1].contig || (x.contig == r[i - 1].contig && x.pos <= r[i - 1].pos))) return RF_ORDER;
+    if (x.kind == K_LIT && (x.src < 0 || x.src + x.prod > lit_bytes)) return RF_LIT;
+    if ((x.kind == K_RAW || x.kind == K_CONV || x.kind == K_RC) && (x.src < 0 || x.src + x.prod > src_end)) return RF_SRC;
+    return RF_OK;
+}
+
 // mutator.py:75-77 as 256-entry tables.
 struct Tables {
     uint8_t conv[256];   // non_ambiguous

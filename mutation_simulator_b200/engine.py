@@ -262,6 +262,15 @@ class Engine:
         nlit = int((recs["src"][recs["kind"] == 2] + recs["prod"][recs["kind"] == 2]).max()) if (recs["kind"] == 2).any() else 0
         self._check(self._lib.ms_load_records(self._h, _ptr(recs), len(recs), _ptr(lit), max(nlit, 0)))
 
+    def load_vcf(self, text, skip_unknown: bool = False) -> bool:
+        """Parse VCF text (bytes-like or mmap, read in place) on the device into the record table (ms_load_vcf).
+        Returns False when the text is not of the regular shape: nothing was loaded and records.records_from_vcf +
+        load_records must take it.  skip_unknown: drop the lines of contigs this engine does not hold."""
+        buf = np.frombuffer(text, dtype=np.uint8) if len(text) else np.zeros(1, np.uint8)
+        reg, n = C.c_int32(0), C.c_int64(0)
+        self._check(self._lib.ms_load_vcf(self._h, _ptr(buf), len(text), int(bool(skip_unknown)), C.byref(reg), C.byref(n)))
+        return bool(reg.value)
+
     def apply(self) -> tuple[int, int]:
         fb, vb = C.c_int64(), C.c_int64()
         self._check(self._lib.ms_apply(self._h, C.byref(fb), C.byref(vb)))

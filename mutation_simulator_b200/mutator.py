@@ -47,7 +47,8 @@ class Mutator:
 
     def load_vcf(self, text):
         """Replay instead of sampling: apply the records of a VCF written by the reference (vcf_writer.py:118-126) or by
-        this package to the same FASTA; mutate() then reproduces that run's *_ms.fa and re-emits the VCF."""
+        this package to the same FASTA; mutate() then reproduces that run's *_ms.fa and re-emits the VCF.  text: str,
+        a bytes-like object or an mmap (parsed in place on the GPU)."""
         self._replay = text
 
     def detach_engine(self):
@@ -93,11 +94,21 @@ class Mutator:
             fasta.upload(eng, my_ids if world > 1 and not tiles else None)
             lap("gather+upload")
             if self._replay is not None:
-                from .records import genome_offsets, records_from_vcf
-                lens = [int(fasta.lengths[g]) for g in my_ids]
-                recs, lit = records_from_vcf(self._replay, [fasta.names[g] for g in my_ids], genome_offsets(lens), lens,
-                                             skip_unknown=world > 1 and not tiles)
-                eng.load_records(recs, lit)
+                # parsed on the device; a VCF of another shape than VcfWriter's goes through the host parser
+                text, skip = self._replay, world > 1 and not tiles
+                if isinstance(text, str):
+                    try:
+                        text = text.encode("latin-1")
+                    except UnicodeEncodeError:
+                        pass
+                if isinstance(text, str) or not eng.load_vcf(text, skip):
+                    from .records import genome_offsets, records_from_vcf
+                    lens = [int(fasta.lengths[g]) for g in my_ids]
+                    if not isinstance(text, (str, bytes, bytearray)):
+                        text = bytes(text)
+                    recs, lit = records_from_vcf(text, [fasta.names[g] for g in my_ids], genome_offsets(lens), lens,
+                                                 skip_unknown=skip)
+                    eng.load_records(recs, lit)
             else:
                 ranges, n = self._planned if (self._planned is not None and len(my_ids) == n_contigs) \
                     else build_ranges(sim, fasta.lengths, my_ids)
@@ -108,7 +119,7 @@ class Mutator:
             else:
                 eng.apply()
             lap("sample+apply")
-            if not args.ignore_warnings and (not tiles or self._rank == 0):
+            if not args.ignore_warnings and (not tiles or self._rank == 0) and getattr(args, "mode", None) != "vcf":
                 per = eng.contig_records()
                 for i in np.flatnonzero(per == 0):
                     print(format_warning(f"No mutations could be generated on sequence {my_ids[int(i)]+1} (mutation rates too low)",
