@@ -209,7 +209,7 @@ int ms_mutate_streamed(ms_ctx* ctx, uint64_t seed, const uint8_t* bases, uint8_t
                        uint8_t* vcf, int64_t vcf_cap, int64_t* fasta_bytes, int64_t* vcf_bytes,
                        int64_t group_min_bases);
 /* which: 0 FASTA image, 1 VCF body, 2 records (ms_rec[]), 3 literal pool, 4 resident genome, 5 BGZF output of the
- * last ms_bgzf_compress */
+ * last ms_bgzf_compress, 6 chain text of the last ms_chain_write */
 int ms_download(ms_ctx* ctx, int which, void* dst, int64_t cap, int64_t* nbytes);
 int ms_device_ptr(ms_ctx* ctx, int which, void** dptr, int64_t* nbytes);
 /* Stream bytes [src_off, src_off+nbytes) of an output buffer into an open file at file_off: D2H through two pinned
@@ -245,8 +245,23 @@ int ms_sample_positions(ms_ctx* ctx, uint64_t seed, int32_t n, const uint32_t* g
  * moving them off the devices (SURVEY.md §4.5: results must not depend on the GPU count). */
 int ms_hash_ranges(ms_ctx* ctx, int which, int32_t n, const int64_t* start, const int64_t* end, uint64_t* out);
 
+/* ---- chain output --------------------------------------------------------
+ * A UCSC chain file (the format liftOver and CrossMap read) from the input genome to the mutated genome of the last
+ * ms_apply or ms_apply_window (which holds the whole table, so every contig is described).  Per contig in FASTA order:
+ * its primary chain, whose aligned blocks are the runs of bases copied unchanged between two base-moving records
+ * (SNPs stay inside blocks), then one single-block chain per record that copies bases from the contig (DU: '+',
+ * forward TLI: '+', IV and reversed TLI: '-' with q on the reverse-complemented mutated contig), in record order.
+ * A contig without a block has no primary chain; a contig without records gets the identity chain.  tName = qName =
+ * the contig name.  ms_chain_count returns the chains of each contig.  ms_chain_write formats the text into buffer 6,
+ * numbering the chains of contig c from first_id[c] (>= 1; ids must stay below 2^31, else MS_ERR_LIMIT), and returns
+ * each contig's slice [chain_off[c], chain_off[c+1]) (n_contigs + 1 entries).  Both return MS_ERR_STATE when no apply
+ * output is current (before an apply, after ms_genome_adopt_output or new records), and MS_ERR_ARG when a copy
+ * record's source leaves its contig. */
+int ms_chain_count(ms_ctx* ctx, int64_t* n_chains /* n_contigs */);
+int ms_chain_write(ms_ctx* ctx, const int64_t* first_id /* n_contigs */, int64_t* chain_off /* n_contigs + 1 */);
+
 /* ---- BGZF output ---------------------------------------------------------
- * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body) into BGZF members on the device; the members,
+ * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body, 6 chain text) into BGZF members on the device; the members,
  * back to back in segment order, become buffer 5 (ms_download, ms_download_to_fd, ms_device_ptr, ms_hash_ranges).
  * Segment s is bytes [src_off[s], src_off[s] + nbytes[s]) of the buffer, followed by one '\n' when add_nl[s] is 1
  * (add_nl may be NULL), and starts at byte file_off[s] of the uncompressed file.  Members never span two segments

@@ -14,6 +14,7 @@ from . import (BedpeWriterError, ChromNotExistError, FastaDuplicateHeaderError, 
                RangeDefinitionOutOfBoundsError, RangeOverlapError, RatesTooHighError, RatesTooLowError, RMTParseError,
                SimulationSettings, TitvTooLowError, VcfWriterError, exit_with_error, get_args, get_md5, load_fasta,
                print_success, print_warning)
+from .chain_writer import ChainWriterError
 from .rmt import MutationSettings
 
 _SETUP_ERRORS = (FileNotFoundError, ITNotEnoughAvailChromsError, RatesTooHighError, RatesTooLowError, FastaIndexingError,
@@ -26,7 +27,8 @@ def check_replay_paths(args):
     """`vcf` mode: the VCF to replay must not be one of the files this run writes (e.g. `-o in vcf in_ms.vcf`), which
     would be truncated before it is read."""
     src = args.vcffile
-    for out in (args.outvcf, args.outfasta):
+    outs = (args.outvcf, args.outfasta) + ((args.outchain,) if getattr(args, "chain", False) else ())
+    for out in outs:
         if out.resolve() == src.resolve() or (out.exists() and src.exists() and os.path.samefile(out, src)):
             raise VcfWriterError(f"The output file {out} would overwrite the input VCF {src}; choose another -o")
 
@@ -110,7 +112,7 @@ def main():
                     fasta.detach_engine()
             mutator.close()
             fasta.close()
-        except (FastaWriterError, VcfWriterError, MutSimError, RangeOverlapError) as e:
+        except (FastaWriterError, VcfWriterError, ChainWriterError, MutSimError, RangeOverlapError) as e:
             exit_with_error(e, args.no_color)
         except ValueError as e:     # a VCF line the replay cannot read (records.records_from_vcf)
             if replay is None:
@@ -130,7 +132,7 @@ def main():
             it_mutator.mutate()
             it_mutator.close()
             fasta.close()
-        except (FastaWriterError, BedpeWriterError, MutSimError) as e:
+        except (FastaWriterError, BedpeWriterError, ChainWriterError, MutSimError) as e:
             exit_with_error(e, args.no_color)
     runtime = round(timer() - start, 4)
     if distributed.rank_world()[0] != 0:

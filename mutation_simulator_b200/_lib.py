@@ -82,6 +82,8 @@ PROTOTYPES = {
     "ms_debug_candidates": (C.c_int, [_P, _I64, _P, _P, _P, _P, C.POINTER(_I64)]),
     "ms_bgzf_compress": (C.c_int, [_P, C.c_int, _I32, _P, _P, _P, _P, _P, C.POINTER(_I64)]),
     "ms_bgzf_compress_host": (C.c_int, [_P, _P, _I64, _P, _I64, C.POINTER(_I64)]),
+    "ms_chain_count": (C.c_int, [_P, _P]),
+    "ms_chain_write": (C.c_int, [_P, _P, _P]),
 }
 
 _lib = None

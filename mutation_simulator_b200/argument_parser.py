@@ -1,8 +1,9 @@
 """Command line of ``mutation-simulator`` — flag for flag the reference's
 (argument_parser.py:31-240) plus three extensions that default to the reference's
 behaviour: ``--seed`` (reproducible runs; default: a fresh random seed, like the
-reference's unseeded RNGs), ``--device`` (CUDA device index) and ``--bgzip``
-(BGZF-compressed FASTA and VCF output, encoded on the GPU), and the ``vcf`` mode
+reference's unseeded RNGs), ``--device`` (CUDA device index), ``--bgzip``
+(BGZF-compressed FASTA and VCF output, encoded on the GPU) and ``--chain`` (a UCSC
+chain file from the input to the mutated genome, built on the GPU), and the ``vcf`` mode
 (replay a VCF the reference or this package wrote onto the same FASTA).
 
 The option table below drives argparse; the derived output names follow
@@ -23,7 +24,7 @@ _PLURAL = {"in": "inserts", "de": "deletions", "iv": "inversion", "du": "duplica
 
 
 def add_outfile_names(args: Namespace) -> Namespace:
-    """outfasta / outfastait / outvcf / outbedpe from the output base."""
+    """outfasta / outfastait / outvcf / outbedpe / outchain / outchainit from the output base."""
     base = args.outbase
     try:
         base = base.with_stem(base.stem + "_ms")
@@ -34,8 +35,10 @@ def add_outfile_names(args: Namespace) -> Namespace:
     args.outfastait = args.outfasta.with_stem(args.outfasta.stem + "_it")
     args.outvcf = args.outfasta.with_suffix(".vcf")
     args.outbedpe = args.outfastait.with_suffix(".bedpe")
-    if getattr(args, "bgzip", False):      # after the derivation: *_it and .bedpe keep their names
-        for k in ("outfasta", "outfastait", "outvcf"):
+    args.outchain = args.outfasta.with_suffix(".chain")
+    args.outchainit = args.outfastait.with_suffix(".chain")
+    if getattr(args, "bgzip", False):      # after the derivation: *_it, .bedpe and .chain keep their names
+        for k in ("outfasta", "outfastait", "outvcf", "outchain", "outchainit"):
             p = getattr(args, k)
             setattr(args, k, p.with_name(p.name + ".gz"))
     return args
@@ -58,6 +61,9 @@ def build_parser() -> ArgumentParser:
     p.add_argument("--device", type=int, default=0, help="[extension] CUDA device index. Default = 0")
     p.add_argument("--bgzip", action="store_true", default=False,
                    help="[extension] write the FASTA and VCF outputs BGZF-compressed (names get .gz); the BEDPE stays plain")
+    p.add_argument("--chain", action="store_true", default=False,
+                   help="[extension] also write a UCSC chain file from the input to the mutated genome (*_ms.chain, "
+                        "*_ms_it.chain for the interchromosomal step; .gz with --bgzip) for liftOver and CrossMap")
 
     sub = p.add_subparsers(dest="mode", help="Generate mutations or interchromosomal translocations via RMT or arguments")
     sub.required = True

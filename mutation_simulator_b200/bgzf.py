@@ -18,10 +18,15 @@ NOT_BGZF = ("Compressed FASTA is only supported in BGZF format. Use the samtools
 
 
 def contig_segments(engine, which: int):
-    """(src_off, nbytes) of every contig's slice of the FASTA image (which=0) or VCF body (which=1) of the last
-    apply(); on one GPU the buffer is the file, so the file offsets are src_off."""
-    fo, vo, _, _ = engine.contig_layout()
-    lay = fo if which == 0 else vo
+    """(src_off, nbytes) of every contig's slice of the FASTA image (which=0), VCF body (which=1) or chain text
+    (which=6, the slices of the last chain_write) of the last apply(); on one GPU the buffer is the file, so the file
+    offsets are src_off."""
+    from .engine import BUF_CHAIN
+    if which == BUF_CHAIN:
+        lay = engine.chain_off
+    else:
+        fo, vo, _, _ = engine.contig_layout()
+        lay = fo if which == 0 else vo
     return lay[:-1].copy(), np.diff(lay)
 
 

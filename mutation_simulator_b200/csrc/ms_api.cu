@@ -33,12 +33,13 @@ void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes) {
     c->counts_valid = false;
     c->sizes_valid = false;
     c->rec_out_valid = true;
+    chain_invalidate(c);
 }
 }  // namespace ms
 
 static const char* STAGE_NAMES[ST_COUNT] = {"upload", "sample_positions", "sample_type_len", "sample_resolve",
                                             "sample_link", "sample_finalize", "plan_scan_layout", "block_index",
-                                            "splice_emit_fasta", "vcf_format", "download"};
+                                            "splice_emit_fasta", "vcf_format", "download", "chain_format"};
 
 extern "C" {
 
@@ -103,7 +104,8 @@ int ms_destroy(ms_ctx* c) {
                       &c->svec, &c->vvec, &c->lvec, &c->tmp_contigs, &c->recs, &c->lit, &c->scan_mid, &c->nvec, &c->sv_stream, &c->snp_stream, &c->piece_lo, &c->piece_desc, &c->fasta, &c->vcf,
                       &c->vcf_off, &c->totals, &c->bucket_range, &c->vend, &c->fa_index, &c->bgzf, &c->bgzf_blocks,
                       &c->bgzf_slots, &c->bgzf_zsize, &c->vp_text, &c->vp_lines, &c->vp_lrec, &c->vp_krec,
-                      &c->vp_lit, &c->vp_names, &c->vp_contig};
+                      &c->vp_lit, &c->vp_names, &c->vp_contig, &c->chain, &c->chain_cc, &c->chain_cons, &c->chain_copy,
+                      &c->chain_off, &c->chain_err};
     for (DevBuf* b : bufs) b->release();
     for (cudaStream_t* s : {&c->s_up, &c->s_down, &c->s_vcf})
         if (*s) { cudaStreamSynchronize(*s); cudaStreamDestroy(*s); }
@@ -185,6 +187,7 @@ static int set_contig_table(ms_ctx* c, int64_t total_bases, int32_t n_contigs, c
     MS_CUDA(c, cudaMemcpyAsync(c->names.p, names, (size_t)name_off[n_contigs], cudaMemcpyHostToDevice, c->stream));
     MS_CUDA(c, cudaStreamSynchronize(c->stream));  // h_contigs / caller buffers may be pageable
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0;
+    chain_invalidate(c);
     return MS_OK;
 }
 
@@ -316,6 +319,7 @@ int ms_genome_subset(ms_ctx* c, const int32_t* ids, int32_t n) {
     MS_CUDA(c, cudaStreamSynchronize(c->stream));
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0; c->sizes_valid = false; c->counts_valid = false;
     c->fasta_bytes = 0; c->vcf_bytes = 0;
+    chain_invalidate(c);
     return MS_OK;
 }
 
@@ -469,6 +473,7 @@ static int which_buffer(ms_ctx* c, int which, void** p, int64_t* n) {
         case 3: *p = c->lit.p; *n = c->lit_bytes; return MS_OK;
         case 4: *p = c->genome.p; *n = c->total_bases; return MS_OK;
         case 5: *p = c->bgzf.p; *n = c->bgzf_bytes; return MS_OK;
+        case 6: *p = c->chain.p; *n = c->chain_bytes; return MS_OK;
         default: MS_FAIL(c, MS_ERR_ARG, "unknown buffer id %d", which);
     }
 }
@@ -636,7 +641,7 @@ int ms_hash_ranges(ms_ctx* c, int which, int32_t n, const int64_t* start, const 
 
 int ms_bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                      const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes) {
-    if (!c || (which != 0 && which != 1) || n_seg < 0 || !total_zbytes ||
+    if (!c || (which != 0 && which != 1 && which != 6) || n_seg < 0 || !total_zbytes ||
         (n_seg > 0 && (!src_off || !nbytes || !file_off || !seg_zbytes)))
         return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
@@ -662,6 +667,18 @@ int ms_bgzf_compress_host(ms_ctx* c, const uint8_t* src, int64_t n, uint8_t* dst
     }
     *zbytes = o;
     return MS_OK;
+}
+
+int ms_chain_count(ms_ctx* c, int64_t* n_chains) {
+    if (!c || !n_chains) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return chain_count(c, n_chains);
+}
+
+int ms_chain_write(ms_ctx* c, const int64_t* first_id, int64_t* chain_off) {
+    if (!c || !first_id || !chain_off) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return chain_write(c, first_id, chain_off);
 }
 
 int ms_get_stats(ms_ctx* c, ms_stats* out) {

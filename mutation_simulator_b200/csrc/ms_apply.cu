@@ -1062,6 +1062,7 @@ int adopt_output(ms_ctx* c) {
     MS_CUDA(c, cudaStreamSynchronize(st));
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0; c->sizes_valid = false; c->counts_valid = false;
     c->fasta_bytes = 0; c->vcf_bytes = 0;
+    chain_invalidate(c);
     return MS_OK;
 }
 
@@ -1074,6 +1075,7 @@ static int plan_stage(ms_ctx* c, bool vcf_sizes) {
     Totals* d_tot = c->totals.as<Totals>();
     cudaStream_t st = c->stream;
 
+    chain_invalidate(c);
     stage_begin(c, ST_PLAN);
     MS_CUDA(c, cudaMemsetAsync(d_tot, 0, sizeof(Totals), st));
     MS_CUDA(c, c->svec.ensure((size_t)(M + 1) * sizeof(int64_t)));
@@ -1239,7 +1241,9 @@ int apply_pipeline(ms_ctx* c) {
     stage_begin(c, ST_VCF);
     if ((rc = vcf_launch(c, 0, c->n_recs, c->stream))) return rc;
     stage_end(c, ST_VCF);
-    return finish_apply(c);
+    if ((rc = finish_apply(c))) return rc;
+    c->chain_ready = true;
+    return MS_OK;
 }
 
 // ---- tile-sharded apply: one genome, several GPUs ------------------------------------------------------------------
@@ -1287,6 +1291,7 @@ int apply_window(ms_ctx* c, int part, int n_parts, int64_t* win) {
         MS_CUDA(c, cudaMemcpyAsync(&v[1], c->vcf_off.as<int64_t>() + r_hi, 8, cudaMemcpyDeviceToHost, c->stream));
     }
     if ((rc = finish_apply(c))) return rc;
+    c->chain_ready = true;
     win[0] = c->fasta_bytes; win[1] = c->vcf_bytes; win[2] = w_lo; win[3] = w_hi; win[4] = v[0]; win[5] = v[1];
     return MS_OK;
 }

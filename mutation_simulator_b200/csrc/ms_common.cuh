@@ -8,6 +8,7 @@
 #include "ms_records.h"
 #include "ms_sample_core.h"
 #include "ms_tile_core.h"
+#include "ms_chain_core.h"
 #include "../../include/mutsim_b200.h"
 
 namespace ms {
@@ -49,7 +50,7 @@ struct Totals {
 };
 
 enum Stage { ST_UPLOAD = 0, ST_SAMPLE_POS, ST_SAMPLE_TYPE, ST_SAMPLE_RESOLVE, ST_SAMPLE_LINK, ST_SAMPLE_FINAL,
-             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_COUNT };
+             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_CHAIN, ST_COUNT };
 
 }  // namespace ms
 
@@ -138,6 +139,13 @@ struct ms_ctx {
     // ms_load_vcf: text, line starts, per-line records (then the new table), compacted records, the new literal pool,
     // the CHROM hash table, scalars and per-contig block bounds
     ms::DevBuf vp_text, vp_lines, vp_lrec, vp_krec, vp_lit, vp_names, vp_contig;
+
+    // chain file of the last apply (buffer 6): per-contig summary, per-SvRec prefixes of cons and of copy records
+    ms::DevBuf chain, chain_cc, chain_cons, chain_copy, chain_off, chain_err;
+    std::vector<ms::ChainCtg> h_chain_cc;
+    int64_t chain_bytes = 0;
+    bool chain_ready = false;     // the SvRec stream and contig table describe the last ms_apply / ms_apply_window
+    bool chain_counted = false;   // h_chain_cc holds ms_chain_count's summary of that output
 };
 
 #define MS_CUDA(ctx, call)                                                                        \
@@ -190,4 +198,7 @@ int record_fault(ms_ctx* c, int fault, int64_t i);
 void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes);
 int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                   const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes);
+void chain_invalidate(ms_ctx* c);
+int chain_count(ms_ctx* c, int64_t* n_chains);
+int chain_write(ms_ctx* c, const int64_t* first_id, int64_t* chain_off);
 }  // namespace ms

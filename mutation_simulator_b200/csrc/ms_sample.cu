@@ -901,6 +901,7 @@ int ms_set_ranges(ms_ctx* c, const ms_range* ranges, int32_t n_ranges, const int
 int ms_sample(ms_ctx* c, uint64_t seed) {
     if (!c) return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
+    chain_invalidate(c);
     return sample_pipeline(c, seed);
 }
 

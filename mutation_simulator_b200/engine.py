@@ -14,7 +14,7 @@ from . import _lib
 from ._lib import MsRange, MsStats, MutSimError
 from .records import REC_DTYPE
 
-BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF = range(6)
+BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF, BUF_CHAIN = range(7)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -315,6 +315,23 @@ class Engine:
         self._check(self._lib.ms_bgzf_compress(self._h, int(which), len(src_off), _ptr(src_off), _ptr(nbytes), _ptr(file_off),
                                                _ptr(nl), _ptr(seg), C.byref(tot)))
         return seg, tot.value
+
+    def chain_count(self) -> np.ndarray:
+        """Chains of each contig in the chain file of the last apply (ms_chain_count)."""
+        out = np.zeros(self.n_contigs, dtype=np.int64)
+        self._check(self._lib.ms_chain_count(self._h, _ptr(out)))
+        return out
+
+    def chain_write(self, first_id) -> np.ndarray:
+        """Format the chain file of the last apply into buffer BUF_CHAIN, numbering contig c's chains from first_id[c]
+        (ms_chain_write).  Returns each contig's slice of the buffer, n_contigs + 1 offsets (kept as chain_off)."""
+        first = np.ascontiguousarray(first_id, dtype=np.int64)
+        if first.size != self.n_contigs:
+            raise ValueError("first_id needs one entry per contig")
+        off = np.zeros(self.n_contigs + 1, dtype=np.int64)
+        self._check(self._lib.ms_chain_write(self._h, _ptr(first), _ptr(off)))
+        self.chain_off = off
+        return off
 
     def fasta(self) -> bytes:
         return self.download(BUF_FASTA).tobytes()

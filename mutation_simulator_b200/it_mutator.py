@@ -50,6 +50,9 @@ class ITMutator:
         if self._world == 1:
             self._fasta_writer = FastaWriter(args.outfastait, getattr(args, "bgzip", False))
             self._bedpe_writer = BedpeWriter(args.outbedpe)
+            if getattr(args, "chain", False):
+                from .chain_writer import write_text
+                write_text(args.outchainit, b"")      # created (and checked) up front like the other outputs
         else:
             self._fasta_writer = self._bedpe_writer = None
         self._seed = D.broadcast_object(run_seed(args))
@@ -84,6 +87,24 @@ class ITMutator:
                 D.barrier()
             self._engine.close()
             self._engine = None
+
+    def _chain_bytes(self, bps) -> bytes:
+        """*_ms_it.chain (BGZF with --bgzip), built on the host from the breakpoints like the BEDPE."""
+        from .chain_writer import encode, it_chain_text
+        fasta = self._fasta
+        text = it_chain_text(list(fasta.names), [int(x) for x in fasta.lengths], self._partners, bps)
+        return encode(text, getattr(self._args, "bgzip", False))
+
+    def _write_chain(self, bps, rank0: bool):
+        """Several GPUs: every rank has all breakpoints; rank 0 writes the file."""
+        if not getattr(self._args, "chain", False):
+            return
+        from .chain_writer import ChainWriterError
+        data = self._chain_bytes(bps) if rank0 else b""
+        try:
+            D.write_partitioned(self._args.outchainit, [0] if rank0 else [], [data] if rank0 else [], 1)
+        except D.OutputCreateError as e:
+            raise ChainWriterError(f"Cannot write to chain file {self._args.outchainit} {e}")
 
     def _pairs_once(self):
         seen, out = set(), []
@@ -170,6 +191,9 @@ class ITMutator:
                 p = self._partners[c]
                 self._bedpe_writer._f.write(rows(fasta[c].name, bps[c]["self"], len(fasta[c]), fasta[p].name,
                                                  bps[c]["partner"], len(fasta[p])))
+        if getattr(self._args, "chain", False):
+            from .chain_writer import write_text
+            write_text(self._args.outchainit, self._chain_bytes(bps))
 
     def _mutate_tiles(self):
         """Fewer (or far more uneven) contigs than GPUs: every rank holds the genome and the same breakpoints (they are
@@ -189,6 +213,7 @@ class ITMutator:
                     p = self._partners[c]
                     bed += rows(fasta[c].name, bps[c]["self"], len(fasta[c]), fasta[p].name, bps[c]["partner"], len(fasta[p]))
         D.write_partitioned(self._args.outbedpe, [0] if rank == 0 else [], [bed] if rank == 0 else [], 1)
+        self._write_chain(bps, rank == 0)
 
     def _mutate_partitioned(self):
         """One process per GPU: contigs are partitioned; for a pair that straddles two GPUs each member reads the
@@ -311,3 +336,4 @@ class ITMutator:
             else:
                 bed.append(b"")
         D.write_partitioned(self._args.outbedpe, my_ids, bed, n_contigs)
+        self._write_chain(bps, self._rank == 0)

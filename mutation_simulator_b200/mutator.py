@@ -43,6 +43,9 @@ class Mutator:
         bgzip = getattr(args, "bgzip", False)
         self._fasta_writer = FastaWriter(args.outfasta, bgzip)
         self._vcf_writer = VcfWriter(args.outvcf, bgzip)
+        if getattr(args, "chain", False):
+            from .chain_writer import write_text
+            write_text(args.outchain, b"")      # created (and checked) up front like the other outputs
         self._vcf_writer.write_header(args.infile.name, fasta, sim.assembly_name, sim.species_name, sim.sample_name)
 
     def load_vcf(self, text):
@@ -124,9 +127,13 @@ class Mutator:
                 for i in np.flatnonzero(per == 0):
                     print(format_warning(f"No mutations could be generated on sequence {my_ids[int(i)]+1} (mutation rates too low)",
                                          args.no_color), file=sys.stderr)
+        chain = getattr(args, "chain", False)
         if world == 1:
             self._fasta_writer.write_from_engine(eng, BUF_FASTA)
             self._vcf_writer.write_from_engine(eng, BUF_VCF)
+            if chain:
+                from .chain_writer import write_from_engine
+                write_from_engine(args.outchain, eng, getattr(args, "bgzip", False))
         else:
             from .fasta_writer import FastaWriterError
             from .vcf_writer import VcfWriterError, header_text
@@ -147,8 +154,33 @@ class Mutator:
                     D.write_slices_partitioned(args.outvcf, eng, BUF_VCF, my_ids, vcf_off, n_contigs, prefix=head, bgzip=bgzip)
             except D.OutputCreateError as e:
                 raise VcfWriterError(f"Cannot write to VCF file {args.outvcf} {e}")
+            if chain:
+                self._write_chain_partitioned(eng, tiles, my_ids, n_contigs, bgzip)
         lap("download+write")
         self.stats = eng.stats() if my_ids else None
         self.host_seconds = {b[0]: b[1] - a[1] for a, b in zip(marks, marks[1:])}
         if os.environ.get("MS_TIMING"):
             print(f"[rank {self._rank}] " + " ".join(f"{k}={v:.3f}s" for k, v in self.host_seconds.items()), file=sys.stderr)
+
+    def _write_chain_partitioned(self, eng, tiles, my_ids, n_contigs, bgzip):
+        """Several GPUs.  Tiles: every rank holds the whole table, formats the whole file and writes its byte window.
+        Contigs: the ranks gather the per-contig chain counts to number the chains, then write their contigs' slices."""
+        from .chain_writer import ChainWriterError, first_ids
+        from .engine import BUF_CHAIN
+        path = self._args.outchain
+        try:
+            if tiles:
+                off = eng.chain_write(first_ids(eng.chain_count()))
+                total = int(off[-1])
+                lo, hi = total * self._rank // self._world, total * (self._rank + 1) // self._world
+                D.write_window(path, eng, BUF_CHAIN, lo, hi, total, bgzip=bgzip)
+            else:
+                mine = eng.chain_count() if my_ids else np.zeros(0, np.int64)
+                counts = np.zeros(n_contigs, dtype=np.int64)
+                for ids, cnt in D.all_gather_object((list(my_ids), [int(x) for x in mine])):
+                    if len(ids):
+                        counts[ids] = cnt
+                off = eng.chain_write(first_ids(counts)[list(my_ids)]) if my_ids else np.zeros(1, np.int64)
+                D.write_slices_partitioned(path, eng, BUF_CHAIN, my_ids, off, n_contigs, bgzip=bgzip)
+        except D.OutputCreateError as e:
+            raise ChainWriterError(f"Cannot write to chain file {path} {e}")
