@@ -209,7 +209,8 @@ int ms_mutate_streamed(ms_ctx* ctx, uint64_t seed, const uint8_t* bases, uint8_t
                        uint8_t* vcf, int64_t vcf_cap, int64_t* fasta_bytes, int64_t* vcf_bytes,
                        int64_t group_min_bases);
 /* which: 0 FASTA image, 1 VCF body, 2 records (ms_rec[]), 3 literal pool, 4 resident genome, 5 BGZF output of the
- * last ms_bgzf_compress, 6 chain text of the last ms_chain_write */
+ * last ms_bgzf_compress, 6 chain text of the last ms_chain_write, 7 phased VCF body of the last ms_vcf_phased,
+ * 8 haplotype masks of the full table */
 int ms_download(ms_ctx* ctx, int which, void* dst, int64_t cap, int64_t* nbytes);
 int ms_device_ptr(ms_ctx* ctx, int which, void** dptr, int64_t* nbytes);
 /* Stream bytes [src_off, src_off+nbytes) of an output buffer into an open file at file_off: D2H through two pinned
@@ -261,7 +262,7 @@ int ms_chain_count(ms_ctx* ctx, int64_t* n_chains /* n_contigs */);
 int ms_chain_write(ms_ctx* ctx, const int64_t* first_id /* n_contigs */, int64_t* chain_off /* n_contigs + 1 */);
 
 /* ---- BGZF output ---------------------------------------------------------
- * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body, 6 chain text) into BGZF members on the device; the members,
+ * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body, 6 chain text, 7 phased VCF body) into BGZF members on the device; the members,
  * back to back in segment order, become buffer 5 (ms_download, ms_download_to_fd, ms_device_ptr, ms_hash_ranges).
  * Segment s is bytes [src_off[s], src_off[s] + nbytes[s]) of the buffer, followed by one '\n' when add_nl[s] is 1
  * (add_nl may be NULL), and starts at byte file_off[s] of the uncompressed file.  Members never span two segments
@@ -275,6 +276,30 @@ int ms_bgzf_compress(ms_ctx* ctx, int which, int32_t n_seg, const int64_t* src_o
 /* The same encoder on the host for small data (the VCF header): src[0..n) as members of 16 KiB each into dst.
  * dst = NULL queries an upper bound of the size.  ctx may be NULL (no device is used). */
 int ms_bgzf_compress_host(ms_ctx* ctx, const uint8_t* src, int64_t n, uint8_t* dst, int64_t cap, int64_t* zbytes);
+
+/* ---- polyploid runs ------------------------------------------------------
+ * A sample of ploidy P (2..8) as P haplotypes of one record table.  Each record of the full table (ms_sample,
+ * ms_load_records, ms_load_vcf*) gets a haplotype mask m, bit h-1 set when haplotype h carries it (buffer 8, one byte
+ * per record).  ms_genotype_draw draws them: blk = Philox(seed, contig gid, purpose 9, key), key = the record's
+ * position, or for a TLI its TL's position (src - contig start), so both halves of a translocation share a mask; the
+ * record is homozygous (m = 2^P - 1) iff blk.x < min(2^32, llround(hom_fraction * 2^32)), else
+ * m = 1 + mulhi32(blk.y, 2^P - 2).  ms_genotype_load takes the masks from the host (n = records of the full table).
+ * ms_load_vcf_phased is ms_load_vcf that also reads the masks from field 10 (GT: exactly P alleles of 0 / 1 joined by
+ * '|'); any other GT gives *regular = 0 like any other irregular line.
+ * ms_select_haplotype(h), h in 1..P, makes the records of haplotype h the active table (compacted on the device; the
+ * literal pool is shared): ms_apply, ms_apply_window, ms_chain_*, ms_contig_layout, ms_contig_records and
+ * ms_download(2) then work on it; like a loaded table, its records carry out = 0 until the next apply.  h = 0 restores
+ * the full table.
+ * ms_vcf_phased formats the VCF body of the full table with the phased GT column (a|b|...) into buffer 7, whichever
+ * haplotype is selected, and returns each contig's slice [vcf_off[c], vcf_off[c+1]) (n_contigs + 1 entries).
+ * MS_ERR_STATE: selecting or formatting without masks (ms_sample, ms_load_*, ms_genome_adopt_output clear them);
+ * MS_ERR_ARG: h > P, P outside 2..8, hom_fraction outside [0, 1]. */
+int ms_genotype_draw(ms_ctx* ctx, uint64_t seed, int32_t ploidy, double hom_fraction);
+int ms_genotype_load(ms_ctx* ctx, const uint8_t* masks, int64_t n, int32_t ploidy);
+int ms_load_vcf_phased(ms_ctx* ctx, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t ploidy,
+                       int32_t* regular, int64_t* n_recs);
+int ms_select_haplotype(ms_ctx* ctx, int32_t h);
+int ms_vcf_phased(ms_ctx* ctx, int64_t* vcf_off /* n_contigs + 1 */);
 
 /* ---- introspection ------------------------------------------------------ */
 int ms_get_stats(ms_ctx* ctx, ms_stats* out);

@@ -27,10 +27,26 @@ def check_replay_paths(args):
     """`vcf` mode: the VCF to replay must not be one of the files this run writes (e.g. `-o in vcf in_ms.vcf`), which
     would be truncated before it is read."""
     src = args.vcffile
-    outs = (args.outvcf, args.outfasta) + ((args.outchain,) if getattr(args, "chain", False) else ())
+    chain = getattr(args, "chain", False)
+    if getattr(args, "ploidy", 1) > 1:       # a polyploid replay writes one FASTA (and chain) per haplotype
+        outs = (args.outvcf, *args.outfastas) + (tuple(args.outchains) if chain else ())
+    else:
+        outs = (args.outvcf, args.outfasta) + ((args.outchain,) if chain else ())
     for out in outs:
         if out.resolve() == src.resolve() or (out.exists() and src.exists() and os.path.samefile(out, src)):
             raise VcfWriterError(f"The output file {out} would overwrite the input VCF {src}; choose another -o")
+
+
+class PloidyError(Exception):
+    """--ploidy >= 2 together with interchromosomal translocations."""
+
+
+def check_ploidy(args, has_it: bool):
+    """A polyploid run has no model for interchromosomal translocations per haplotype: `it` mode, or an RMT with an IT
+    section, together with --ploidy >= 2 is refused before any output file is opened."""
+    if getattr(args, "ploidy", 1) > 1 and has_it:
+        raise PloidyError(f"--ploidy {args.ploidy} cannot be combined with interchromosomal translocations "
+                          "(it mode or an RMT with an IT section); run them with --ploidy 1")
 
 
 def read_replay_vcf(path):
@@ -47,11 +63,12 @@ def read_replay_vcf(path):
 
 def initialize():
     args = get_args()
-    if args.mode == "vcf":      # before any output file is opened
-        try:
+    try:                        # before any output file is opened
+        check_ploidy(args, args.mode == "it")
+        if args.mode == "vcf":
             check_replay_paths(args)
-        except VcfWriterError as e:
-            exit_with_error(e, args.no_color)
+    except (VcfWriterError, PloidyError) as e:
+        exit_with_error(e, args.no_color)
     try:
         from . import distributed
         # the file is parsed on the GPU and stays there for the engines (SURVEY.md §8 f1); with several GPUs every
@@ -67,7 +84,8 @@ def initialize():
             sim = SimulationSettings.from_rmt(args.rmtfile, fasta, args.ignore_warnings)
         else:   # vcf: the records come from the file; no ranges, no IT
             sim = SimulationSettings(MutationSettings(None, None), None, [], None, ignore_warnings=args.ignore_warnings)
-    except _SETUP_ERRORS + (MutSimError,) as e:   # MutSimError: no usable CUDA device / library (there is no CPU fallback)
+        check_ploidy(args, sim.has_it)
+    except _SETUP_ERRORS + (MutSimError, PloidyError) as e:   # MutSimError: no usable CUDA device / library (there is no CPU fallback)
         exit_with_error(e, args.no_color)
     if not args.ignore_warnings:
         warn_user(args, sim)

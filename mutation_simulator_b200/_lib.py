@@ -84,6 +84,11 @@ PROTOTYPES = {
     "ms_bgzf_compress_host": (C.c_int, [_P, _P, _I64, _P, _I64, C.POINTER(_I64)]),
     "ms_chain_count": (C.c_int, [_P, _P]),
     "ms_chain_write": (C.c_int, [_P, _P, _P]),
+    "ms_genotype_draw": (C.c_int, [_P, _U64, _I32, C.c_double]),
+    "ms_genotype_load": (C.c_int, [_P, _P, _I64, _I32]),
+    "ms_load_vcf_phased": (C.c_int, [_P, _P, _I64, _I32, _I32, C.POINTER(_I32), C.POINTER(_I64)]),
+    "ms_select_haplotype": (C.c_int, [_P, _I32]),
+    "ms_vcf_phased": (C.c_int, [_P, _P]),
 }
 
 _lib = None

@@ -2,15 +2,23 @@
 (argument_parser.py:31-240) plus three extensions that default to the reference's
 behaviour: ``--seed`` (reproducible runs; default: a fresh random seed, like the
 reference's unseeded RNGs), ``--device`` (CUDA device index), ``--bgzip``
-(BGZF-compressed FASTA and VCF output, encoded on the GPU) and ``--chain`` (a UCSC
-chain file from the input to the mutated genome, built on the GPU), and the ``vcf`` mode
-(replay a VCF the reference or this package wrote onto the same FASTA).
+(BGZF-compressed FASTA and VCF output, encoded on the GPU), ``--chain`` (a UCSC
+chain file from the input to the mutated genome, built on the GPU) and ``--ploidy`` /
+``--hom-fraction`` (a diploid or polyploid sample: one FASTA per haplotype and a phased
+VCF, genotypes drawn on the GPU), and the ``vcf`` mode (replay a VCF the reference or
+this package wrote onto the same FASTA).
+
+With ``--ploidy P`` >= 2 the record table is sampled as for one haplotype; each record then
+carries haplotype h with a drawn genotype: homozygous (on all P haplotypes) with probability
+``--hom-fraction``, else on a uniformly drawn non-empty proper subset of them.  The run writes
+``*_ms_h1.fa`` .. ``*_ms_hP.fa`` (and ``*_ms_h1.chain`` .. with ``--chain``) instead of
+``*_ms.fa``, and one phased ``*_ms.vcf`` (GT ``1|0``, ``0|1``, ``1|1``, ...).
 
 The option table below drives argparse; the derived output names follow
 argument_parser.py:14-28."""
 from __future__ import annotations
 
-from argparse import ArgumentParser, Namespace
+from argparse import ArgumentParser, ArgumentTypeError, Namespace
 from pathlib import Path
 
 from ._version import __version__
@@ -24,7 +32,8 @@ _PLURAL = {"in": "inserts", "de": "deletions", "iv": "inversion", "du": "duplica
 
 
 def add_outfile_names(args: Namespace) -> Namespace:
-    """outfasta / outfastait / outvcf / outbedpe / outchain / outchainit from the output base."""
+    """outfasta / outfastait / outvcf / outbedpe / outchain / outchainit from the output base; outfastas / outchains:
+    the per-haplotype FASTA and chain files of a polyploid run (empty lists for ploidy 1)."""
     base = args.outbase
     try:
         base = base.with_stem(base.stem + "_ms")
@@ -37,11 +46,33 @@ def add_outfile_names(args: Namespace) -> Namespace:
     args.outbedpe = args.outfastait.with_suffix(".bedpe")
     args.outchain = args.outfasta.with_suffix(".chain")
     args.outchainit = args.outfastait.with_suffix(".chain")
+    hap = range(1, getattr(args, "ploidy", 1) + 1) if getattr(args, "ploidy", 1) > 1 else ()
+    args.outfastas = [args.outfasta.with_stem(f"{args.outfasta.stem}_h{h}") for h in hap]
+    args.outchains = [args.outchain.with_stem(f"{args.outchain.stem}_h{h}") for h in hap]
     if getattr(args, "bgzip", False):      # after the derivation: *_it, .bedpe and .chain keep their names
         for k in ("outfasta", "outfastait", "outvcf", "outchain", "outchainit"):
             p = getattr(args, k)
             setattr(args, k, p.with_name(p.name + ".gz"))
+        args.outfastas = [p.with_name(p.name + ".gz") for p in args.outfastas]
+        args.outchains = [p.with_name(p.name + ".gz") for p in args.outchains]
     return args
+
+
+MAX_PLOIDY = 8
+
+
+def _ploidy(text: str) -> int:
+    v = int(text)
+    if not 1 <= v <= MAX_PLOIDY:
+        raise ArgumentTypeError(f"ploidy must be between 1 and {MAX_PLOIDY}, got {v}")
+    return v
+
+
+def _fraction(text: str) -> float:
+    v = float(text)
+    if not 0.0 <= v <= 1.0:
+        raise ArgumentTypeError(f"hom-fraction must be between 0 and 1, got {text}")
+    return v
 
 
 def build_parser() -> ArgumentParser:
@@ -64,6 +95,12 @@ def build_parser() -> ArgumentParser:
     p.add_argument("--chain", action="store_true", default=False,
                    help="[extension] also write a UCSC chain file from the input to the mutated genome (*_ms.chain, "
                         "*_ms_it.chain for the interchromosomal step; .gz with --bgzip) for liftOver and CrossMap")
+    p.add_argument("--ploidy", type=_ploidy, default=D.PLOIDY,
+                   help=f"[extension] haplotypes of the simulated sample (1..{MAX_PLOIDY}); >= 2 writes *_ms_h1.fa .. *_ms_hP.fa and a "
+                        f"phased *_ms.vcf, and in vcf mode reads the GT of a phased VCF. Default = {D.PLOIDY}")
+    p.add_argument("--hom-fraction", type=_fraction, default=D.HOM_FRACTION, dest="hom_fraction",
+                   help=f"[extension] probability that a record of a polyploid sample is on every haplotype (homozygous); "
+                        f"the others go to a uniformly drawn proper subset. Default = {D.HOM_FRACTION}")
 
     sub = p.add_subparsers(dest="mode", help="Generate mutations or interchromosomal translocations via RMT or arguments")
     sub.required = True

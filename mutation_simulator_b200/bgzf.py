@@ -18,12 +18,14 @@ NOT_BGZF = ("Compressed FASTA is only supported in BGZF format. Use the samtools
 
 
 def contig_segments(engine, which: int):
-    """(src_off, nbytes) of every contig's slice of the FASTA image (which=0), VCF body (which=1) or chain text
-    (which=6, the slices of the last chain_write) of the last apply(); on one GPU the buffer is the file, so the file
-    offsets are src_off."""
-    from .engine import BUF_CHAIN
+    """(src_off, nbytes) of every contig's slice of the FASTA image (which=0), VCF body (which=1), chain text
+    (which=6, the slices of the last chain_write) or phased VCF body (which=7, those of the last vcf_phased) of the last
+    apply(); on one GPU the buffer is the file, so the file offsets are src_off."""
+    from .engine import BUF_CHAIN, BUF_VCF_PHASED
     if which == BUF_CHAIN:
         lay = engine.chain_off
+    elif which == BUF_VCF_PHASED:
+        lay = engine.vcf_phased_off
     else:
         fo, vo, _, _ = engine.contig_layout()
         lay = fo if which == 0 else vo

@@ -10,6 +10,7 @@
 #include <sys/statvfs.h>
 #include "ms_bgzf_core.h"
 #include "ms_common.cuh"
+#include "ms_genotype_core.h"
 
 using namespace ms;
 
@@ -34,12 +35,14 @@ void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes) {
     c->sizes_valid = false;
     c->rec_out_valid = true;
     chain_invalidate(c);
+    genotype_clear(c);
 }
 }  // namespace ms
 
 static const char* STAGE_NAMES[ST_COUNT] = {"upload", "sample_positions", "sample_type_len", "sample_resolve",
                                             "sample_link", "sample_finalize", "plan_scan_layout", "block_index",
-                                            "splice_emit_fasta", "vcf_format", "download", "chain_format"};
+                                            "splice_emit_fasta", "vcf_format", "download", "chain_format",
+                                            "genotype", "select", "vcf_phased"};
 
 extern "C" {
 
@@ -105,7 +108,8 @@ int ms_destroy(ms_ctx* c) {
                       &c->vcf_off, &c->totals, &c->bucket_range, &c->vend, &c->fa_index, &c->bgzf, &c->bgzf_blocks,
                       &c->bgzf_slots, &c->bgzf_zsize, &c->vp_text, &c->vp_lines, &c->vp_lrec, &c->vp_krec,
                       &c->vp_lit, &c->vp_names, &c->vp_contig, &c->chain, &c->chain_cc, &c->chain_cons, &c->chain_copy,
-                      &c->chain_off, &c->chain_err};
+                      &c->chain_off, &c->chain_err, &c->gt_mask, &c->recs_full, &c->gt_vcf, &c->gt_voff, &c->gt_ctg_off,
+                      &c->vp_lmask, &c->vp_kmask};
     for (DevBuf* b : bufs) b->release();
     for (cudaStream_t* s : {&c->s_up, &c->s_down, &c->s_vcf})
         if (*s) { cudaStreamSynchronize(*s); cudaStreamDestroy(*s); }
@@ -188,6 +192,7 @@ static int set_contig_table(ms_ctx* c, int64_t total_bases, int32_t n_contigs, c
     MS_CUDA(c, cudaStreamSynchronize(c->stream));  // h_contigs / caller buffers may be pageable
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0;
     chain_invalidate(c);
+    genotype_clear(c);
     return MS_OK;
 }
 
@@ -237,6 +242,7 @@ int ms_mutate_streamed(ms_ctx* c, uint64_t seed, const uint8_t* bases, uint8_t* 
                        int64_t vcf_cap, int64_t* fasta_bytes, int64_t* vcf_bytes, int64_t group_min_bases) {
     if (!c || !bases || !fasta || !vcf) return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
+    genotype_clear(c);
     const int rc = mutate_streamed(c, seed, bases, fasta, fasta_cap, vcf, vcf_cap, fasta_bytes, vcf_bytes, group_min_bases);
     if (rc != MS_OK) {   // nothing may still be copying from / into the caller's buffers when the error is reported
         cudaStreamSynchronize(c->stream);
@@ -320,6 +326,7 @@ int ms_genome_subset(ms_ctx* c, const int32_t* ids, int32_t n) {
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0; c->sizes_valid = false; c->counts_valid = false;
     c->fasta_bytes = 0; c->vcf_bytes = 0;
     chain_invalidate(c);
+    genotype_clear(c);
     return MS_OK;
 }
 
@@ -444,7 +451,42 @@ int ms_load_vcf(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unk
     *regular = 0; *n_recs = 0;
     if (c->n_contigs <= 0) MS_FAIL(c, MS_ERR_STATE, "ms_load_vcf: upload a genome first");
     MS_CUDA(c, cudaSetDevice(c->device));
-    return vcf_load(c, text, nbytes, skip_unknown, regular, n_recs);
+    return vcf_load(c, text, nbytes, skip_unknown, 0, regular, n_recs);
+}
+
+int ms_load_vcf_phased(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t ploidy, int32_t* regular,
+                       int64_t* n_recs) {
+    if (!c || nbytes < 0 || (nbytes > 0 && !text) || !regular || !n_recs) return MS_ERR_ARG;
+    *regular = 0; *n_recs = 0;
+    if (ploidy < 2 || ploidy > MAX_PLOIDY) MS_FAIL(c, MS_ERR_ARG, "ms_load_vcf_phased: ploidy %d outside 2..%d", ploidy, MAX_PLOIDY);
+    if (c->n_contigs <= 0) MS_FAIL(c, MS_ERR_STATE, "ms_load_vcf_phased: upload a genome first");
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return vcf_load(c, text, nbytes, skip_unknown, ploidy, regular, n_recs);
+}
+
+// ---- polyploid runs -------------------------------------------------------------------
+int ms_genotype_draw(ms_ctx* c, uint64_t seed, int32_t ploidy, double hom_fraction) {
+    if (!c) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return genotype_draw(c, seed, ploidy, hom_fraction);
+}
+
+int ms_genotype_load(ms_ctx* c, const uint8_t* masks, int64_t n, int32_t ploidy) {
+    if (!c || n < 0 || (n > 0 && !masks)) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return genotype_load(c, masks, n, ploidy);
+}
+
+int ms_select_haplotype(ms_ctx* c, int32_t h) {
+    if (!c) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return select_haplotype(c, h);
+}
+
+int ms_vcf_phased(ms_ctx* c, int64_t* vcf_off) {
+    if (!c || !vcf_off) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return vcf_phased(c, vcf_off);
 }
 
 // ---- apply ----------------------------------------------------------------------------
@@ -474,6 +516,8 @@ static int which_buffer(ms_ctx* c, int which, void** p, int64_t* n) {
         case 4: *p = c->genome.p; *n = c->total_bases; return MS_OK;
         case 5: *p = c->bgzf.p; *n = c->bgzf_bytes; return MS_OK;
         case 6: *p = c->chain.p; *n = c->chain_bytes; return MS_OK;
+        case 7: *p = c->gt_vcf.p; *n = c->gt_vcf_bytes; return MS_OK;
+        case 8: *p = c->gt_mask.p; *n = c->gt_ploidy ? (c->gt_selected ? c->gt_n_full : c->n_recs) : 0; return MS_OK;
         default: MS_FAIL(c, MS_ERR_ARG, "unknown buffer id %d", which);
     }
 }
@@ -641,7 +685,7 @@ int ms_hash_ranges(ms_ctx* c, int which, int32_t n, const int64_t* start, const 
 
 int ms_bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                      const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes) {
-    if (!c || (which != 0 && which != 1 && which != 6) || n_seg < 0 || !total_zbytes ||
+    if (!c || (which != 0 && which != 1 && which != 6 && which != 7) || n_seg < 0 || !total_zbytes ||
         (n_seg > 0 && (!src_off || !nbytes || !file_off || !seg_zbytes)))
         return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));

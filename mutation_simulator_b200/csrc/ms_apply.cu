@@ -1063,6 +1063,7 @@ int adopt_output(ms_ctx* c) {
     c->n_recs = 0; c->lit_bytes = 0; c->n_ranges = 0; c->sizes_valid = false; c->counts_valid = false;
     c->fasta_bytes = 0; c->vcf_bytes = 0;
     chain_invalidate(c);
+    genotype_clear(c);
     return MS_OK;
 }
 

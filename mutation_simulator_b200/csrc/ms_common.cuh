@@ -50,7 +50,7 @@ struct Totals {
 };
 
 enum Stage { ST_UPLOAD = 0, ST_SAMPLE_POS, ST_SAMPLE_TYPE, ST_SAMPLE_RESOLVE, ST_SAMPLE_LINK, ST_SAMPLE_FINAL,
-             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_CHAIN, ST_COUNT };
+             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_CHAIN, ST_GENOTYPE, ST_SELECT, ST_VCF_PHASED, ST_COUNT };
 
 }  // namespace ms
 
@@ -146,6 +146,15 @@ struct ms_ctx {
     int64_t chain_bytes = 0;
     bool chain_ready = false;     // the SvRec stream and contig table describe the last ms_apply / ms_apply_window
     bool chain_counted = false;   // h_chain_cc holds ms_chain_count's summary of that output
+
+    // polyploid runs (ms_genotype.cu): haplotype masks of the full table (buffer 8), the full table while a haplotype's
+    // records are the active table, the phased VCF body (buffer 7), its per-record and per-contig offsets
+    ms::DevBuf gt_mask, recs_full, gt_vcf, gt_voff, gt_ctg_off, vp_lmask, vp_kmask;
+    int32_t gt_ploidy = 0;        // 0: the current table has no masks
+    int32_t gt_selected = 0;      // haplotype whose records are the active table (0: the full table is)
+    int64_t gt_n_full = 0;        // records of the full table while a haplotype is selected
+    bool gt_sizes_valid_full = false;
+    int64_t gt_vcf_bytes = 0;
 };
 
 #define MS_CUDA(ctx, call)                                                                        \
@@ -193,7 +202,8 @@ int mutate_streamed(ms_ctx* c, uint64_t seed, const uint8_t* h_bases, uint8_t* h
 int count_types(ms_ctx* c);
 int fill_record_out(ms_ctx* c);
 int hash_ranges(ms_ctx* c, const uint8_t* buf, int32_t n, const int64_t* start, const int64_t* end, uint64_t* out);
-int vcf_load(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t* regular, int64_t* n_recs);
+int vcf_load(ms_ctx* c, const uint8_t* text, int64_t nbytes, int32_t skip_unknown, int32_t ploidy, int32_t* regular,
+             int64_t* n_recs);
 int record_fault(ms_ctx* c, int fault, int64_t i);
 void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes);
 int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
@@ -201,4 +211,9 @@ int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, c
 void chain_invalidate(ms_ctx* c);
 int chain_count(ms_ctx* c, int64_t* n_chains);
 int chain_write(ms_ctx* c, const int64_t* first_id, int64_t* chain_off);
+void genotype_clear(ms_ctx* c);
+int genotype_draw(ms_ctx* c, uint64_t seed, int32_t ploidy, double hom_fraction);
+int genotype_load(ms_ctx* c, const uint8_t* masks, int64_t n, int32_t ploidy);
+int select_haplotype(ms_ctx* c, int32_t h);
+int vcf_phased(ms_ctx* c, int64_t* vcf_off);
 }  // namespace ms

@@ -67,6 +67,7 @@ enum Purpose : uint32_t {
     P_TL_REV    = 6,   // inversion coin of one translocation                       (mutator.py:307-316)
     P_IT_KEY    = 7,   // the same for the breakpoint ranges of an interchromosomal pair (it_mutator.py:94-118)
     P_GENOME    = 8,   // synthetic genome generator (bench only)
+    P_GENOTYPE  = 9,   // haplotype mask of one record of a polyploid run (ms_genotype_core.h)
 };
 
 struct Seed { uint32_t k0, k1; };

@@ -902,6 +902,7 @@ int ms_sample(ms_ctx* c, uint64_t seed) {
     if (!c) return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
     chain_invalidate(c);
+    genotype_clear(c);
     return sample_pipeline(c, seed);
 }
 

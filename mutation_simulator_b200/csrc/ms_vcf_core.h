@@ -103,8 +103,14 @@ template <class S> MS_HD void put_info(S& s, const char* sv, int svn, uint32_t e
     put_str(s, ";SVLEN=", 7); put_uint(s, len);
 }
 
-// Emits the whole line (caller has checked vcf_omitted).
-template <class S> MS_HD void vcf_emit(S& s, const VcfView& v, const Contig& c, const Rec& r) {
+// the GT column of a haploid line (K7's)
+struct HaploidGt {
+    template <class S> MS_HD void operator()(S& s) const { put_str(s, "\tGT\t1\n", 6); }
+};
+
+// Emits the whole line (caller has checked vcf_omitted); gt writes everything from the tab before FORMAT on
+// (ms_genotype_core.h's PhasedGt for a polyploid run).
+template <class S, class Gt = HaploidGt> MS_HD void vcf_emit(S& s, const VcfView& v, const Contig& c, const Rec& r, Gt gt = Gt()) {
     const int64_t g0 = c.goff;
     const uint32_t p = r.pos;
     if constexpr (S::counting) s.skip((uint32_t)c.name_len);
@@ -159,7 +165,7 @@ template <class S> MS_HD void vcf_emit(S& s, const VcfView& v, const Contig& c, 
     }
     put_str(s, "\t.\t.\t", 5);
     if (r.type == T_SN) s.put('.'); else put_info(s, sv, svn, end, svlen);
-    put_str(s, "\tGT\t1\n", 6);
+    gt(s);
 }
 
 // Size of the line vcf_emit() writes, in closed form (the sampler sizes 40 M records per genome: running the

@@ -75,6 +75,23 @@ __global__ void __launch_bounds__(256) k_vcf_place(const Rec* krec, int64_t m, c
     recs[base[r.contig] + j] = r;
 }
 
+// ms_load_vcf_phased: the haplotype mask of every record line from its GT field (other lines keep 0)
+__global__ void __launch_bounds__(256)
+k_vcf_parse_gt(const uint8_t* t, const int64_t* lines, int64_t n_lines, const Rec* lrec, int ploidy, uint8_t* lmask, int* irregular) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n_lines) return;
+    uint8_t m = 0;
+    if (lrec[k].type != T_DEAD && !parse_gt(t, lines[k], lines[k + 1] - 1, ploidy, &m)) *irregular = 1;
+    lmask[k] = m;
+}
+
+// the masks follow their records to the table order of k_vcf_place
+__global__ void __launch_bounds__(256) k_vcf_place_mask(const Rec* krec, const uint8_t* kmask, int64_t m, const int64_t* base, uint8_t* mask) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= m) return;
+    mask[base[krec[j].contig] + j] = kmask[j];
+}
+
 // the first record that fails a check of ms_load_records: (index << 3) | RecFault
 __global__ void __launch_bounds__(256)
 k_vcf_faults(const Rec* recs, int64_t m, int32_t n_contigs, int64_t lit_bytes, int64_t src_end, unsigned long long* first) {
@@ -84,7 +101,7 @@ k_vcf_faults(const Rec* recs, int64_t m, int32_t n_contigs, int64_t lit_bytes, i
     if (f) atomicMin(first, ((unsigned long long)j << 3) | (unsigned long long)f);
 }
 
-int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, int32_t* regular, int64_t* n_recs) {
+int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, int32_t ploidy, int32_t* regular, int64_t* n_recs) {
     cudaStream_t st = c->stream;
     const int32_t nc = c->n_contigs;
 
@@ -156,12 +173,24 @@ int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, in
     Rec* lrec = c->vp_lrec.as<Rec>();
     Rec* krec = c->vp_krec.as<Rec>();
     uint8_t* pool = c->vp_lit.as<uint8_t>();
+    uint8_t* lmask = nullptr;    // ploidy > 0: masks per line, then per compacted record
+    uint8_t* kmask = nullptr;
+    if (ploidy > 0) {
+        MS_CUDA(c, c->vp_lmask.ensure((size_t)n_lines + 16));
+        MS_CUDA(c, c->vp_kmask.ensure((size_t)n_lines + 16));
+        lmask = c->vp_lmask.as<uint8_t>();
+        kmask = c->vp_kmask.as<uint8_t>();
+    }
     I64x2 tot{0, 0};
     int h_irr = 0;
     if (n_lines > 0) {
         const int64_t* lines = c->vp_lines.as<int64_t>();
         k_vcf_parse_lines<<<(unsigned)ceil_div(n_lines, 256), 256, 0, st>>>(t, lines, n_lines, names, skip_unknown, lrec, d_irr);
         MS_LAUNCH_CHECK(c);
+        if (lmask) {
+            k_vcf_parse_gt<<<(unsigned)ceil_div(n_lines, 256), 256, 0, st>>>(t, lines, n_lines, lrec, ploidy, lmask, d_irr);
+            MS_LAUNCH_CHECK(c);
+        }
         auto in = [=] __device__(int64_t k) -> I64x2 {
             const Rec& r = lrec[k];
             return r.type == T_DEAD ? I64x2{0, 0} : I64x2{1, r.kind == K_LIT ? (int64_t)r.prod : 0};
@@ -174,6 +203,7 @@ int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, in
                 r.src = ex.b;
             }
             krec[ex.a] = r;
+            if (lmask) kmask[ex.a] = lmask[k];
         };
         I64x2* d_tot = nullptr;
         MS_CUDA(c, device_scan<I64x2>(c, in, out, n_lines, I64x2{0, 0}, SumOp(), c->scan_tmp, &d_tot));
@@ -202,6 +232,10 @@ int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, in
         MS_CUDA(c, cudaMemcpyAsync(d_base, base.data(), (size_t)nc * 8, cudaMemcpyHostToDevice, st));
         k_vcf_place<<<grid, 256, 0, st>>>(krec, m, d_base, lrec);
         MS_LAUNCH_CHECK(c);
+        if (lmask) {
+            k_vcf_place_mask<<<grid, 256, 0, st>>>(krec, kmask, m, d_base, lmask);
+            MS_LAUNCH_CHECK(c);
+        }
         k_vcf_faults<<<grid, 256, 0, st>>>(lrec, m, nc, lit_bytes, c->total_bases + 64 + c->foreign_cap, d_fault);
         MS_LAUNCH_CHECK(c);
         // (a K_RAW source in a peer window, which ms_load_records accepts, cannot come from a VCF line: its sources
@@ -214,6 +248,10 @@ int vcf_load(ms_ctx* c, const uint8_t* text, int64_t n, int32_t skip_unknown, in
     std::swap(c->recs, c->vp_lrec);
     std::swap(c->lit, c->vp_lit);
     records_loaded(c, m, lit_bytes);
+    if (ploidy > 0) {
+        std::swap(c->gt_mask, c->vp_lmask);
+        c->gt_ploidy = ploidy;
+    }
     *regular = 1;
     *n_recs = m;
     return MS_OK;

@@ -190,5 +190,27 @@ MS_HD int parse_line(const uint8_t* t, int64_t lo, int64_t hi, const NameTable& 
     return VL_REC;
 }
 
+// The phased genotype of a record line [lo, hi) (ms_load_vcf_phased): field 10 (up to the next tab or the line end)
+// must be exactly `ploidy` alleles from {0, 1} joined by '|'.  *mask gets bit h-1 for allele h = 1.  false: the line is
+// IRREGULAR (records.records_from_vcf with `ploidy` owns the message).
+MS_HD bool parse_gt(const uint8_t* t, int64_t lo, int64_t hi, int ploidy, uint8_t* mask) {
+    int64_t g = lo;
+    for (int tabs = 0; tabs < 9; ++g) {
+        if (g >= hi) return false;      // fewer than 10 fields
+        if (t[g] == '\t') ++tabs;
+    }
+    int64_t e = g;
+    while (e < hi && t[e] != '\t') ++e;
+    if (e - g != 2 * (int64_t)ploidy - 1) return false;
+    uint32_t m = 0;
+    for (int h = 0; h < ploidy; ++h) {
+        const uint8_t a = t[g + 2 * h];
+        if ((a != '0' && a != '1') || (h && t[g + 2 * h - 1] != '|')) return false;
+        m |= (uint32_t)(a - '0') << h;
+    }
+    *mask = (uint8_t)m;
+    return true;
+}
+
 }  // namespace vcfp
 }  // namespace ms

@@ -19,6 +19,10 @@ class Defaults:
     BLOCK = 1
     MINLEN, MAXLEN = 1, 2
     IV_MINLEN, IV_MAXLEN = 2, 3
+    # extensions: one haploid sample; for a polyploid one, about the het:hom-alt ratio of 1.5-2 usually seen in one
+    # human sample (a documented default, not a measured claim)
+    PLOIDY = 1
+    HOM_FRACTION = 0.35
 
 
 Defaults.MUT_BLOCK = {t: Defaults.BLOCK for t in (MutType.SN, MutType.IN, MutType.DE, MutType.IV, MutType.DU, MutType.TL, MutType.TLI)}

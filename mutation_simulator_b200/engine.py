@@ -14,7 +14,7 @@ from . import _lib
 from ._lib import MsRange, MsStats, MutSimError
 from .records import REC_DTYPE
 
-BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF, BUF_CHAIN = range(7)
+BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF, BUF_CHAIN, BUF_VCF_PHASED, BUF_GT = range(9)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -270,6 +270,41 @@ class Engine:
         reg, n = C.c_int32(0), C.c_int64(0)
         self._check(self._lib.ms_load_vcf(self._h, _ptr(buf), len(text), int(bool(skip_unknown)), C.byref(reg), C.byref(n)))
         return bool(reg.value)
+
+    def load_vcf_phased(self, text, ploidy: int, skip_unknown: bool = False) -> bool:
+        """load_vcf that also reads each record's haplotype mask from its GT field (ms_load_vcf_phased).  False: the text
+        (a GT included) is not of the regular shape and records.records_from_vcf(..., ploidy=) must take it."""
+        buf = np.frombuffer(text, dtype=np.uint8) if len(text) else np.zeros(1, np.uint8)
+        reg, n = C.c_int32(0), C.c_int64(0)
+        self._check(self._lib.ms_load_vcf_phased(self._h, _ptr(buf), len(text), int(bool(skip_unknown)), int(ploidy), C.byref(reg),
+                                                 C.byref(n)))
+        return bool(reg.value)
+
+    # -- polyploid runs ----------------------------------------------------
+    def genotype_draw(self, seed: int, ploidy: int, hom_fraction: float):
+        """Draw the haplotype mask of every record of the full table (ms_genotype_draw)."""
+        self._check(self._lib.ms_genotype_draw(self._h, C.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), int(ploidy), float(hom_fraction)))
+
+    def genotype_load(self, masks, ploidy: int):
+        """Host-supplied haplotype masks, one per record of the full table (ms_genotype_load)."""
+        m = np.ascontiguousarray(masks, dtype=np.uint8)
+        self._check(self._lib.ms_genotype_load(self._h, _ptr(m) if m.size else None, int(m.size), int(ploidy)))
+
+    def select_haplotype(self, h: int):
+        """Make haplotype h's records (1..P) the active table; 0 restores the full table (ms_select_haplotype)."""
+        self._check(self._lib.ms_select_haplotype(self._h, int(h)))
+
+    def vcf_phased(self) -> np.ndarray:
+        """Format the phased VCF body of the full table into buffer BUF_VCF_PHASED (ms_vcf_phased).  Returns each
+        contig's slice, n_contigs + 1 offsets (kept as vcf_phased_off)."""
+        off = np.zeros(self.n_contigs + 1, dtype=np.int64)
+        self._check(self._lib.ms_vcf_phased(self._h, _ptr(off)))
+        self.vcf_phased_off = off
+        return off
+
+    def genotypes(self) -> np.ndarray:
+        """Haplotype masks of the full table (bit h-1: haplotype h carries the record)."""
+        return self.download(BUF_GT)
 
     def apply(self) -> tuple[int, int]:
         fb, vb = C.c_int64(), C.c_int64()

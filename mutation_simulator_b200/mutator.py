@@ -3,7 +3,11 @@
 ``Mutator(args, fasta, sim).mutate()`` samples positions, types and lengths for every
 range of every contig, resolves overlaps, links translocations, splices the genome and
 formats FASTA + VCF — all on the GPU through libmutsim_b200 — then writes the two files.
-Nothing here touches a base on the host."""
+Nothing here touches a base on the host.
+
+With ``--ploidy P`` >= 2 the same table is sampled, every record draws its haplotype mask on the GPU, the phased VCF of
+the whole table is written, and then each haplotype's records are selected on the device and applied in turn: one
+FASTA (and chain) per haplotype."""
 from __future__ import annotations
 
 import os
@@ -14,7 +18,7 @@ import time
 import numpy as np
 
 from . import distributed as D
-from .engine import BUF_FASTA, BUF_VCF, Engine
+from .engine import BUF_FASTA, BUF_VCF, BUF_VCF_PHASED, Engine
 from .fasta_writer import FastaWriter
 from .plan import block_list, build_ranges, p_transition
 from .util import format_warning
@@ -34,6 +38,8 @@ class Mutator:
         self._engine = None
         self.stats = None
         self._replay = None
+        self._ploidy = getattr(args, "ploidy", 1)
+        self._hap_writers = []
         # plan the ranges (and reject overlapping ones) BEFORE any output file is opened and truncated: a settings
         # error must not leave partial *_ms.fa / *_ms.vcf behind (the reference dies later, with both files cut)
         self._planned = build_ranges(sim, fasta.lengths, None) if sim.has_mutations else None
@@ -41,11 +47,16 @@ class Mutator:
             self._fasta_writer = self._vcf_writer = None
             return
         bgzip = getattr(args, "bgzip", False)
-        self._fasta_writer = FastaWriter(args.outfasta, bgzip)
+        if self._ploidy > 1:     # one FASTA per haplotype instead of *_ms.fa
+            self._fasta_writer = None
+            self._hap_writers = [FastaWriter(p, bgzip) for p in args.outfastas]
+        else:
+            self._fasta_writer = FastaWriter(args.outfasta, bgzip)
         self._vcf_writer = VcfWriter(args.outvcf, bgzip)
         if getattr(args, "chain", False):
             from .chain_writer import write_text
-            write_text(args.outchain, b"")      # created (and checked) up front like the other outputs
+            for p in (args.outchains if self._ploidy > 1 else [args.outchain]):
+                write_text(p, b"")      # created (and checked) up front like the other outputs
         self._vcf_writer.write_header(args.infile.name, fasta, sim.assembly_name, sim.species_name, sim.sample_name)
 
     def load_vcf(self, text):
@@ -61,8 +72,11 @@ class Mutator:
         return eng
 
     def close(self):
+        for w in self._hap_writers:
+            w.close()
         if self._fasta_writer is not None:
             self._fasta_writer.close()
+        if self._vcf_writer is not None:
             self._vcf_writer.close()
         if self._engine is not None:
             self._engine.close()
@@ -104,29 +118,38 @@ class Mutator:
                         text = text.encode("latin-1")
                     except UnicodeEncodeError:
                         pass
-                if isinstance(text, str) or not eng.load_vcf(text, skip):
+                ploidy = self._ploidy if self._ploidy > 1 else None
+                loaded = not isinstance(text, str) and \
+                    (eng.load_vcf_phased(text, ploidy, skip) if ploidy else eng.load_vcf(text, skip))
+                if not loaded:
                     from .records import genome_offsets, records_from_vcf
                     lens = [int(fasta.lengths[g]) for g in my_ids]
                     if not isinstance(text, (str, bytes, bytearray)):
                         text = bytes(text)
-                    recs, lit = records_from_vcf(text, [fasta.names[g] for g in my_ids], genome_offsets(lens), lens,
-                                                 skip_unknown=skip)
+                    recs, lit, *masks = records_from_vcf(text, [fasta.names[g] for g in my_ids], genome_offsets(lens), lens,
+                                                         skip_unknown=skip, ploidy=ploidy)
                     eng.load_records(recs, lit)
+                    if ploidy:
+                        eng.genotype_load(masks[0], ploidy)
             else:
                 ranges, n = self._planned if (self._planned is not None and len(my_ids) == n_contigs) \
                     else build_ranges(sim, fasta.lengths, my_ids)
                 eng.set_ranges_array(ranges, n, block_list(sim), min(sim.mut_block.values()), p_transition(sim.titv))
                 eng.sample(seed)
-            if tiles:
+                if self._ploidy > 1:
+                    eng.genotype_draw(seed, self._ploidy, getattr(args, "hom_fraction", 0.35))
+            if self._ploidy > 1:
+                eng.vcf_phased()
+            elif tiles:
                 window = eng.apply_window(self._rank, world)
             else:
                 eng.apply()
             lap("sample+apply")
-            if not args.ignore_warnings and (not tiles or self._rank == 0) and getattr(args, "mode", None) != "vcf":
-                per = eng.contig_records()
-                for i in np.flatnonzero(per == 0):
-                    print(format_warning(f"No mutations could be generated on sequence {my_ids[int(i)]+1} (mutation rates too low)",
-                                         args.no_color), file=sys.stderr)
+            if self._ploidy == 1 and not args.ignore_warnings and (not tiles or self._rank == 0) \
+                    and getattr(args, "mode", None) != "vcf":      # (a polyploid run warns after its haplotypes)
+                self._warn_empty(eng.contig_records(), my_ids)
+        if self._ploidy > 1:
+            return self._mutate_haplotypes(eng, tiles, my_ids, n_contigs, lap, marks)
         chain = getattr(args, "chain", False)
         if world == 1:
             self._fasta_writer.write_from_engine(eng, BUF_FASTA)
@@ -157,17 +180,80 @@ class Mutator:
             if chain:
                 self._write_chain_partitioned(eng, tiles, my_ids, n_contigs, bgzip)
         lap("download+write")
+        self._finish(eng, my_ids, marks)
+
+    def _finish(self, eng, my_ids, marks):
         self.stats = eng.stats() if my_ids else None
         self.host_seconds = {b[0]: b[1] - a[1] for a, b in zip(marks, marks[1:])}
         if os.environ.get("MS_TIMING"):
             print(f"[rank {self._rank}] " + " ".join(f"{k}={v:.3f}s" for k, v in self.host_seconds.items()), file=sys.stderr)
 
-    def _write_chain_partitioned(self, eng, tiles, my_ids, n_contigs, bgzip):
+    def _mutate_haplotypes(self, eng, tiles, my_ids, n_contigs, lap, marks):
+        """Polyploid run, after the table and its genotypes are in place and the phased VCF is formatted: write the VCF,
+        then select, apply and write each haplotype in turn.  Several GPUs: in contig mode each rank writes its contigs'
+        slices (ms_vcf_phased's per-contig offsets); in tile mode every rank formatted the whole VCF and writes its byte
+        window, and applies its window of each haplotype."""
+        args, fasta, sim = self._args, self._fasta, self._sim
+        world, bgzip, chain = self._world, getattr(args, "bgzip", False), getattr(args, "chain", False)
+        from .fasta_writer import FastaWriterError
+        from .vcf_writer import VcfWriterError
+        if world == 1:
+            self._vcf_writer.write_from_engine(eng, BUF_VCF_PHASED)
+        else:
+            from .vcf_writer import header_text
+            head = header_text(args.infile.name, [(fasta[k].name, len(fasta[k])) for k in fasta.keys()], sim.assembly_name,
+                               sim.species_name, sim.sample_name).encode("latin-1")
+            off = eng.vcf_phased_off if my_ids else np.zeros(1, np.int64)
+            try:
+                if tiles:
+                    total = int(off[-1])
+                    D.write_window(args.outvcf, eng, BUF_VCF_PHASED, total * self._rank // world,
+                                   total * (self._rank + 1) // world, total, prefix=head, bgzip=bgzip)
+                else:
+                    D.write_slices_partitioned(args.outvcf, eng, BUF_VCF_PHASED, my_ids, off, n_contigs, prefix=head, bgzip=bgzip)
+            except D.OutputCreateError as e:
+                raise VcfWriterError(f"Cannot write to VCF file {args.outvcf} {e}")
+        per = np.zeros(len(my_ids), dtype=np.int64)
+        for h in range(1, self._ploidy + 1):
+            path = args.outfastas[h - 1]
+            if my_ids:
+                eng.select_haplotype(h)
+                window = eng.apply_window(self._rank, world) if tiles else None
+                if not tiles:
+                    eng.apply()
+                per += eng.contig_records()
+            try:
+                if world == 1:
+                    self._hap_writers[h - 1].write_from_engine(eng, BUF_FASTA)
+                elif tiles:
+                    D.write_window(path, eng, BUF_FASTA, *window["fasta"], window["fasta_bytes"], bgzip=bgzip)
+                else:
+                    D.write_fasta_partitioned(path, eng, my_ids, n_contigs, bgzip=bgzip)
+            except D.OutputCreateError as e:
+                raise FastaWriterError(f"Cannot write to Fasta file {path} {e}")
+            if chain:
+                if world == 1:
+                    from .chain_writer import write_from_engine
+                    write_from_engine(args.outchains[h - 1], eng, bgzip)
+                else:
+                    self._write_chain_partitioned(eng, tiles, my_ids, n_contigs, bgzip, args.outchains[h - 1])
+        lap("haplotypes")
+        if my_ids and not args.ignore_warnings and (not tiles or self._rank == 0) and getattr(args, "mode", None) != "vcf":
+            self._warn_empty(per, my_ids)        # a contig that no haplotype mutates got no records at all
+        self._finish(eng, my_ids, marks)
+
+    def _warn_empty(self, per_contig, my_ids):
+        for i in np.flatnonzero(per_contig == 0):
+            print(format_warning(f"No mutations could be generated on sequence {my_ids[int(i)]+1} (mutation rates too low)",
+                                 self._args.no_color), file=sys.stderr)
+
+    def _write_chain_partitioned(self, eng, tiles, my_ids, n_contigs, bgzip, path=None):
         """Several GPUs.  Tiles: every rank holds the whole table, formats the whole file and writes its byte window.
-        Contigs: the ranks gather the per-contig chain counts to number the chains, then write their contigs' slices."""
+        Contigs: the ranks gather the per-contig chain counts to number the chains, then write their contigs' slices.
+        path: the chain file (default *_ms.chain; a polyploid run writes one per haplotype)."""
         from .chain_writer import ChainWriterError, first_ids
         from .engine import BUF_CHAIN
-        path = self._args.outchain
+        path = path or self._args.outchain
         try:
             if tiles:
                 off = eng.chain_write(first_ids(eng.chain_count()))

@@ -116,8 +116,19 @@ def _get(m, name, default=KeyError):
 _SVTYPE = {"INS": T_IN, "DEL": T_DE, "INV": T_IV, "DUP": T_DU, "DEL:ME": T_TL, "INS:ME": T_TLI}
 
 
-def records_from_vcf(text, names, goff, lengths, skip_unknown: bool = False) -> tuple[np.ndarray, np.ndarray]:
+def parse_gt(field: str, ploidy: int) -> int:
+    """A phased genotype of `ploidy` alleles from {0, 1} joined by '|' -> its haplotype mask (bit h-1 = allele h is 1);
+    ValueError for anything else."""
+    alleles = field.split("|")
+    if len(alleles) != ploidy or any(a not in ("0", "1") for a in alleles):
+        raise ValueError(f"GT {field!r} is not a phased genotype of ploidy {ploidy} ({ploidy} alleles of 0 or 1 joined by '|')")
+    return sum(1 << h for h, a in enumerate(alleles) if a == "1")
+
+
+def records_from_vcf(text, names, goff, lengths, skip_unknown: bool = False, ploidy=None):
     """VCF text (header lines are skipped) -> (recs sorted by (contig, pos), literal pool) for ``ms_load_records``.
+    With `ploidy` (a phased VCF of a polyploid run) -> (recs, literal pool, haplotype masks in record order): field 10 of
+    every record must be a GT of exactly `ploidy` alleles of 0 / 1 joined by '|' (:func:`parse_gt`).
 
     names: contig names (VCF CHROM) in genome order; goff/lengths as in :func:`build_records`.
     The replay rule is "replace REF by ALT at POS" (SURVEY.md §8c) expressed without touching the anchor base of
@@ -135,7 +146,7 @@ def records_from_vcf(text, names, goff, lengths, skip_unknown: bool = False) -> 
     if isinstance(text, (bytes, bytearray)):
         text = bytes(text).decode("latin-1")
     index = {(n.decode("latin-1") if isinstance(n, (bytes, bytearray)) else str(n)): i for i, n in enumerate(names)}
-    rows, lit = [], bytearray()
+    rows, lit, masks = [], bytearray(), {}
     for ln, line in enumerate(text.splitlines(), 1):
         if not line or line[0] == "#":
             continue
@@ -147,6 +158,13 @@ def records_from_vcf(text, names, goff, lengths, skip_unknown: bool = False) -> 
                 continue
             raise ValueError(f"VCF line {ln}: unknown contig {f[0]!r}")
         ci = index[f[0]]
+        if ploidy is not None:
+            if len(f) < 10:
+                raise ValueError(f"VCF line {ln}: no GT field (field 10) for ploidy {ploidy}")
+            try:
+                masks[len(rows)] = parse_gt(f[9], ploidy)
+            except ValueError as e:
+                raise ValueError(f"VCF line {ln}: {e}") from None
         g0, L = int(goff[ci]), int(lengths[ci])
         pos1, ref, alt = int(f[1]), f[3].encode("latin-1"), f[4].encode("latin-1")
         if f[7] == ".":
@@ -186,6 +204,10 @@ def records_from_vcf(text, names, goff, lengths, skip_unknown: bool = False) -> 
         p, c = rows[-1][0], rows[-1][1]
         if not (0 <= p < L) or p + c > L:
             raise ValueError(f"VCF line {ln}: record outside contig {f[0]!r} (length {L})")
-    rows.sort(key=lambda r: (r[9], r[0]))
+    order = sorted(range(len(rows)), key=lambda i: (rows[i][9], rows[i][0]))
+    rows = [rows[i] for i in order]
     recs = np.array(rows, dtype=REC_DTYPE) if rows else np.zeros(0, dtype=REC_DTYPE)
-    return recs, np.frombuffer(bytes(lit) + b"\0" * 16, dtype=np.uint8).copy()
+    pool = np.frombuffer(bytes(lit) + b"\0" * 16, dtype=np.uint8).copy()
+    if ploidy is None:
+        return recs, pool
+    return recs, pool, np.array([masks[i] for i in order], dtype=np.uint8)
