@@ -210,7 +210,7 @@ int ms_mutate_streamed(ms_ctx* ctx, uint64_t seed, const uint8_t* bases, uint8_t
                        int64_t group_min_bases);
 /* which: 0 FASTA image, 1 VCF body, 2 records (ms_rec[]), 3 literal pool, 4 resident genome, 5 BGZF output of the
  * last ms_bgzf_compress, 6 chain text of the last ms_chain_write, 7 phased VCF body of the last ms_vcf_phased,
- * 8 haplotype masks of the full table */
+ * 8 haplotype masks of the full table, 9 FASTQ records of the last ms_reads_write */
 int ms_download(ms_ctx* ctx, int which, void* dst, int64_t cap, int64_t* nbytes);
 int ms_device_ptr(ms_ctx* ctx, int which, void** dptr, int64_t* nbytes);
 /* Stream bytes [src_off, src_off+nbytes) of an output buffer into an open file at file_off: D2H through two pinned
@@ -262,7 +262,7 @@ int ms_chain_count(ms_ctx* ctx, int64_t* n_chains /* n_contigs */);
 int ms_chain_write(ms_ctx* ctx, const int64_t* first_id /* n_contigs */, int64_t* chain_off /* n_contigs + 1 */);
 
 /* ---- BGZF output ---------------------------------------------------------
- * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body, 6 chain text, 7 phased VCF body) into BGZF members on the device; the members,
+ * Compresses segments of buffer `which` (0 FASTA image, 1 VCF body, 6 chain text, 7 phased VCF body, 9 FASTQ records) into BGZF members on the device; the members,
  * back to back in segment order, become buffer 5 (ms_download, ms_download_to_fd, ms_device_ptr, ms_hash_ranges).
  * Segment s is bytes [src_off[s], src_off[s] + nbytes[s]) of the buffer, followed by one '\n' when add_nl[s] is 1
  * (add_nl may be NULL), and starts at byte file_off[s] of the uncompressed file.  Members never span two segments
@@ -300,6 +300,37 @@ int ms_load_vcf_phased(ms_ctx* ctx, const uint8_t* text, int64_t nbytes, int32_t
                        int32_t* regular, int64_t* n_recs);
 int ms_select_haplotype(ms_ctx* ctx, int32_t h);
 int ms_vcf_phased(ms_ctx* ctx, int64_t* vcf_off /* n_contigs + 1 */);
+
+/* ---- paired-end reads ----------------------------------------------------
+ * Read pairs drawn from the mutated genome of the active table's last FULL ms_apply (buffer 0 and the records' out
+ * positions), as FASTQ records.  Pair i of contig c (gid g, mutated length Lp >= read_len) on haplotype cfg->hap is a
+ * pure function of (seed, g, hap, i): attempt a = 0..7 reads the words of Philox blocks (g, purpose 10 | hap << 8 |
+ * b << 12, i * 16 + a), b = 0, 1, ...; fragment f = frag_mean + ((frag_sd * (w0 + ... + w11 - 6 * 2^32) + 2^31) >> 32)
+ * clamped to [read_len, Lp], start s = mulhi32(w12, Lp - f + 1), strand '-' iff bit 0 of w13; an attempt whose two
+ * template ends hold a byte other than A/C/G/T is redrawn, the 8th is kept.  '+': R1 = [s, s + L) forward, R2 = the
+ * reverse complement of [s + f - L, s + f); '-' swaps them.  Base j of R1 (R2) becomes a substitution iff word
+ * 16 + j (16 + L + j) is below llround(error_rate * 2^32), and then the (word mod 3)-th other base in ACGT order.
+ * Record: "@name:hap:i:s+1:f:strand:lift(x1)+1:lift(x2)+1/1\n" (x1, x2 = leftmost template base of R1, R2; '*'
+ * where it lifts to no input base along the primary chain), the bases, "\n+\n", read_len times qual, "\n".  R2
+ * records are the same with "/2" and have the same size.
+ * pairs are numbered contig-major over the context's contigs: pair j of contig c = sum(n_pairs[<c]) + j.
+ * ms_reads_size returns in bytes[c] the bytes one file's records of pairs [first, first + count) take in contig c
+ * (n_contigs entries).  ms_reads_write formats those pairs: R1 records at [0, nbytes) of buffer 9, R2 records at
+ * [nbytes, 2 * nbytes); right after ms_reads_size of the same range it reuses that call's draws.
+ * MS_ERR_STATE when no full apply output is current (before an apply, after ms_apply_window, ms_genome_adopt_output
+ * or new records); MS_ERR_ARG for a cfg outside hap 1..8, read_len 1..1000, frag_mean read_len..10^6, frag_sd
+ * 0..10^5, 0 <= error_rate < 1, qual 33..126, a negative n_pairs, pairs on a contig shorter than read_len, or a range
+ * past the total. */
+typedef struct {
+    uint64_t seed;
+    int32_t hap, read_len, frag_mean, frag_sd;
+    double error_rate;
+    uint8_t qual;
+} ms_reads_cfg;
+int ms_reads_size(ms_ctx* ctx, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count,
+                  int64_t* bytes /* n_contigs */);
+int ms_reads_write(ms_ctx* ctx, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count,
+                   int64_t* nbytes);
 
 /* ---- introspection ------------------------------------------------------ */
 int ms_get_stats(ms_ctx* ctx, ms_stats* out);

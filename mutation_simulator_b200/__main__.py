@@ -15,6 +15,7 @@ from . import (BedpeWriterError, ChromNotExistError, FastaDuplicateHeaderError, 
                SimulationSettings, TitvTooLowError, VcfWriterError, exit_with_error, get_args, get_md5, load_fasta,
                print_success, print_warning)
 from .chain_writer import ChainWriterError
+from .reads_writer import ReadsWriterError
 from .rmt import MutationSettings
 
 _SETUP_ERRORS = (FileNotFoundError, ITNotEnoughAvailChromsError, RatesTooHighError, RatesTooLowError, FastaIndexingError,
@@ -32,6 +33,8 @@ def check_replay_paths(args):
         outs = (args.outvcf, *args.outfastas) + (tuple(args.outchains) if chain else ())
     else:
         outs = (args.outvcf, args.outfasta) + ((args.outchain,) if chain else ())
+    if getattr(args, "reads", None) is not None:
+        outs += (args.outreads1, args.outreads2)
     for out in outs:
         if out.resolve() == src.resolve() or (out.exists() and src.exists() and os.path.samefile(out, src)):
             raise VcfWriterError(f"The output file {out} would overwrite the input VCF {src}; choose another -o")
@@ -47,6 +50,19 @@ def check_ploidy(args, has_it: bool):
     if getattr(args, "ploidy", 1) > 1 and has_it:
         raise PloidyError(f"--ploidy {args.ploidy} cannot be combined with interchromosomal translocations "
                           "(it mode or an RMT with an IT section); run them with --ploidy 1")
+
+
+class ReadsError(Exception):
+    """--reads together with interchromosomal translocations."""
+
+
+def check_reads(args, has_it: bool):
+    """Reads are drawn from the first step's mutated genome, and their names give positions on it and on the input:
+    `it` mode, or an RMT with an IT section, together with --reads is refused before any output file is opened, since
+    the reads would have to come from the IT step's genome while their truth names the first step's."""
+    if getattr(args, "reads", None) is not None and has_it:
+        raise ReadsError("--reads cannot be combined with interchromosomal translocations (it mode or an RMT with an IT "
+                         "section); the reads would come from the IT genome while their truth names the first step's genome")
 
 
 def read_replay_vcf(path):
@@ -65,9 +81,10 @@ def initialize():
     args = get_args()
     try:                        # before any output file is opened
         check_ploidy(args, args.mode == "it")
+        check_reads(args, args.mode == "it")
         if args.mode == "vcf":
             check_replay_paths(args)
-    except (VcfWriterError, PloidyError) as e:
+    except (VcfWriterError, PloidyError, ReadsError) as e:
         exit_with_error(e, args.no_color)
     try:
         from . import distributed
@@ -85,7 +102,8 @@ def initialize():
         else:   # vcf: the records come from the file; no ranges, no IT
             sim = SimulationSettings(MutationSettings(None, None), None, [], None, ignore_warnings=args.ignore_warnings)
         check_ploidy(args, sim.has_it)
-    except _SETUP_ERRORS + (MutSimError, PloidyError) as e:   # MutSimError: no usable CUDA device / library (there is no CPU fallback)
+        check_reads(args, sim.has_it)
+    except _SETUP_ERRORS + (MutSimError, PloidyError, ReadsError) as e:   # MutSimError: no usable CUDA device / library (there is no CPU fallback)
         exit_with_error(e, args.no_color)
     if not args.ignore_warnings:
         warn_user(args, sim)
@@ -130,7 +148,7 @@ def main():
                     fasta.detach_engine()
             mutator.close()
             fasta.close()
-        except (FastaWriterError, VcfWriterError, ChainWriterError, MutSimError, RangeOverlapError) as e:
+        except (FastaWriterError, VcfWriterError, ChainWriterError, ReadsWriterError, MutSimError, RangeOverlapError) as e:
             exit_with_error(e, args.no_color)
         except ValueError as e:     # a VCF line the replay cannot read (records.records_from_vcf)
             if replay is None:

@@ -32,6 +32,11 @@ class MsStats(C.Structure):
                 ("kernel_launches", C.c_int64), ("counts", C.c_int64 * 8), ("stage_ms", C.c_float * 16)]
 
 
+class MsReadsCfg(C.Structure):
+    _fields_ = [("seed", C.c_uint64), ("hap", C.c_int32), ("read_len", C.c_int32), ("frag_mean", C.c_int32),
+                ("frag_sd", C.c_int32), ("error_rate", C.c_double), ("qual", C.c_uint8)]
+
+
 MS_OK, MS_ERR_CUDA, MS_ERR_ARG, MS_ERR_STATE, MS_ERR_SAMPLE, MS_ERR_OVERLAP, MS_ERR_LIMIT, MS_ERR_INTERNAL = range(8)
 
 _P, _I64, _I32, _U64, _U32 = C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint32
@@ -89,6 +94,8 @@ PROTOTYPES = {
     "ms_load_vcf_phased": (C.c_int, [_P, _P, _I64, _I32, _I32, C.POINTER(_I32), C.POINTER(_I64)]),
     "ms_select_haplotype": (C.c_int, [_P, _I32]),
     "ms_vcf_phased": (C.c_int, [_P, _P]),
+    "ms_reads_size": (C.c_int, [_P, C.POINTER(MsReadsCfg), _P, _I64, _I64, _P]),
+    "ms_reads_write": (C.c_int, [_P, C.POINTER(MsReadsCfg), _P, _I64, _I64, C.POINTER(_I64)]),
 }
 
 _lib = None

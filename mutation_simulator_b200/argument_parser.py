@@ -5,8 +5,9 @@ reference's unseeded RNGs), ``--device`` (CUDA device index), ``--bgzip``
 (BGZF-compressed FASTA and VCF output, encoded on the GPU), ``--chain`` (a UCSC
 chain file from the input to the mutated genome, built on the GPU) and ``--ploidy`` /
 ``--hom-fraction`` (a diploid or polyploid sample: one FASTA per haplotype and a phased
-VCF, genotypes drawn on the GPU), and the ``vcf`` mode (replay a VCF the reference or
-this package wrote onto the same FASTA).
+VCF, genotypes drawn on the GPU), ``--reads`` (paired-end reads of the mutated sample,
+drawn on the GPU), and the ``vcf`` mode (replay a VCF the reference or this package wrote
+onto the same FASTA).
 
 With ``--ploidy P`` >= 2 the record table is sampled as for one haplotype; each record then
 carries haplotype h with a drawn genotype: homozygous (on all P haplotypes) with probability
@@ -14,11 +15,18 @@ carries haplotype h with a drawn genotype: homozygous (on all P haplotypes) with
 ``*_ms_h1.fa`` .. ``*_ms_hP.fa`` (and ``*_ms_h1.chain`` .. with ``--chain``) instead of
 ``*_ms.fa``, and one phased ``*_ms.vcf`` (GT ``1|0``, ``0|1``, ``1|1``, ...).
 
+With ``--reads C`` each haplotype gets C / P of the sample's mean depth as read pairs
+(``--read-length``, ``--fragment-mean``, ``--fragment-sd``, ``--read-error-rate``), written
+to ``*_ms_R1.fq`` and ``*_ms_R2.fq`` next to ``*_ms.vcf``; every read name carries the pair's
+position on the mutated contig and where its reads start on the input genome.  The read
+options are ignored (and absent from the namespace) without ``--reads``.
+
 The option table below drives argparse; the derived output names follow
 argument_parser.py:14-28."""
 from __future__ import annotations
 
-from argparse import ArgumentParser, ArgumentTypeError, Namespace
+import math
+from argparse import SUPPRESS, ArgumentParser, ArgumentTypeError, Namespace
 from pathlib import Path
 
 from ._version import __version__
@@ -49,12 +57,16 @@ def add_outfile_names(args: Namespace) -> Namespace:
     hap = range(1, getattr(args, "ploidy", 1) + 1) if getattr(args, "ploidy", 1) > 1 else ()
     args.outfastas = [args.outfasta.with_stem(f"{args.outfasta.stem}_h{h}") for h in hap]
     args.outchains = [args.outchain.with_stem(f"{args.outchain.stem}_h{h}") for h in hap]
+    if getattr(args, "reads", None) is not None:
+        args.outreads1, args.outreads2 = (args.outvcf.with_name(f"{args.outvcf.stem}_R{m}.fq") for m in (1, 2))
     if getattr(args, "bgzip", False):      # after the derivation: *_it, .bedpe and .chain keep their names
         for k in ("outfasta", "outfastait", "outvcf", "outchain", "outchainit"):
             p = getattr(args, k)
             setattr(args, k, p.with_name(p.name + ".gz"))
         args.outfastas = [p.with_name(p.name + ".gz") for p in args.outfastas]
         args.outchains = [p.with_name(p.name + ".gz") for p in args.outchains]
+        if getattr(args, "reads", None) is not None:
+            args.outreads1, args.outreads2 = (p.with_name(p.name + ".gz") for p in (args.outreads1, args.outreads2))
     return args
 
 
@@ -73,6 +85,31 @@ def _fraction(text: str) -> float:
     if not 0.0 <= v <= 1.0:
         raise ArgumentTypeError(f"hom-fraction must be between 0 and 1, got {text}")
     return v
+
+
+# --reads options: (flag, dest, type, default, lowest, highest or None, help); checked only when --reads is given
+_READS = [("--read-length", "read_length", int, D.READ_LENGTH, 1, 1000, "bases per read"),
+          ("--fragment-mean", "fragment_mean", int, D.FRAGMENT_MEAN, None, 1_000_000,
+           "mean fragment (insert) length, from the read length"),
+          ("--fragment-sd", "fragment_sd", int, D.FRAGMENT_SD, 0, 100_000, "fragment length standard deviation"),
+          ("--read-error-rate", "read_error_rate", float, D.READ_ERROR_RATE, 0.0, None, "per-base substitution error rate, below 1")]
+
+
+def _check_reads(p: ArgumentParser, args: Namespace):
+    """Fill in the read options' defaults and check them; exits with status 2 like any argparse error."""
+    if not (math.isfinite(args.reads) and args.reads > 0):
+        p.error(f"argument --reads: the depth must be finite and > 0, got {args.reads}")
+    for flag, dest, typ, default, lo, hi, _ in _READS:
+        v = getattr(args, dest, default)
+        try:                    # taken as text by argparse, so that without --reads nothing about them is checked
+            v = typ(v)
+        except ValueError:
+            p.error(f"argument {flag}: invalid {typ.__name__} value: {v!r}")
+        setattr(args, dest, v)
+        lo = args.read_length if dest == "fragment_mean" else lo
+        if v < lo or (hi is not None and v > hi) or (dest == "read_error_rate" and not v < 1.0):
+            top = "below 1" if hi is None else f"at most {hi}"
+            p.error(f"argument {flag}: must be at least {lo} and {top}, got {v}")
 
 
 def build_parser() -> ArgumentParser:
@@ -101,6 +138,11 @@ def build_parser() -> ArgumentParser:
     p.add_argument("--hom-fraction", type=_fraction, default=D.HOM_FRACTION, dest="hom_fraction",
                    help=f"[extension] probability that a record of a polyploid sample is on every haplotype (homozygous); "
                         f"the others go to a uniformly drawn proper subset. Default = {D.HOM_FRACTION}")
+    p.add_argument("--reads", type=float, default=SUPPRESS, metavar="C",
+                   help="[extension] also simulate paired-end reads of the mutated sample at mean depth C (each haplotype "
+                        "gets C / ploidy) into *_ms_R1.fq and *_ms_R2.fq (.gz with --bgzip), with the truth in every read name")
+    for flag, dest, typ, default, _, _, hlp in _READS:
+        p.add_argument(flag, dest=dest, default=SUPPRESS, help=f"[extension] with --reads: {hlp}. Default = {default}")
 
     sub = p.add_subparsers(dest="mode", help="Generate mutations or interchromosomal translocations via RMT or arguments")
     sub.required = True
@@ -130,7 +172,14 @@ def build_parser() -> ArgumentParser:
 
 
 def get_args(argv=None) -> Namespace:
-    args = build_parser().parse_args(argv)
+    p = build_parser()
+    args = p.parse_args(argv)
+    if hasattr(args, "reads"):
+        _check_reads(p, args)
+    else:                       # the read options mean nothing without --reads
+        for _, dest, *_ in _READS:
+            if hasattr(args, dest):
+                delattr(args, dest)
     if args.quiet:
         args.ignore_warnings = True
         args.no_progress = True

@@ -15,7 +15,7 @@ CSRC = PKG / "csrc"
 OBJ = PKG / "_obj"
 LIB = PKG / "libmutsim_b200.so"
 SOURCES = ["ms_api.cu", "ms_apply.cu", "ms_sample.cu", "ms_genome.cu", "ms_ingest.cu", "ms_bgzf.cu", "ms_vcf_parse.cu", "ms_chain.cu",
-           "ms_genotype.cu"]
+           "ms_genotype.cu", "ms_reads.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
               "--extended-lambda", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-Wall", "-Xcudafe", "--diag_suppress=177"]

@@ -42,7 +42,7 @@ void records_loaded(ms_ctx* c, int64_t n_recs, int64_t lit_bytes) {
 static const char* STAGE_NAMES[ST_COUNT] = {"upload", "sample_positions", "sample_type_len", "sample_resolve",
                                             "sample_link", "sample_finalize", "plan_scan_layout", "block_index",
                                             "splice_emit_fasta", "vcf_format", "download", "chain_format",
-                                            "genotype", "select", "vcf_phased"};
+                                            "genotype", "select", "vcf_phased", "reads"};
 
 extern "C" {
 
@@ -109,7 +109,7 @@ int ms_destroy(ms_ctx* c) {
                       &c->bgzf_slots, &c->bgzf_zsize, &c->vp_text, &c->vp_lines, &c->vp_lrec, &c->vp_krec,
                       &c->vp_lit, &c->vp_names, &c->vp_contig, &c->chain, &c->chain_cc, &c->chain_cons, &c->chain_copy,
                       &c->chain_off, &c->chain_err, &c->gt_mask, &c->recs_full, &c->gt_vcf, &c->gt_voff, &c->gt_ctg_off,
-                      &c->vp_lmask, &c->vp_kmask};
+                      &c->vp_lmask, &c->vp_kmask, &c->reads, &c->reads_info, &c->reads_off, &c->reads_pre, &c->reads_ctg};
     for (DevBuf* b : bufs) b->release();
     for (cudaStream_t* s : {&c->s_up, &c->s_down, &c->s_vcf})
         if (*s) { cudaStreamSynchronize(*s); cudaStreamDestroy(*s); }
@@ -518,6 +518,7 @@ static int which_buffer(ms_ctx* c, int which, void** p, int64_t* n) {
         case 6: *p = c->chain.p; *n = c->chain_bytes; return MS_OK;
         case 7: *p = c->gt_vcf.p; *n = c->gt_vcf_bytes; return MS_OK;
         case 8: *p = c->gt_mask.p; *n = c->gt_ploidy ? (c->gt_selected ? c->gt_n_full : c->n_recs) : 0; return MS_OK;
+        case 9: *p = c->reads.p; *n = c->reads_bytes; return MS_OK;
         default: MS_FAIL(c, MS_ERR_ARG, "unknown buffer id %d", which);
     }
 }
@@ -685,7 +686,7 @@ int ms_hash_ranges(ms_ctx* c, int which, int32_t n, const int64_t* start, const 
 
 int ms_bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                      const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes) {
-    if (!c || (which != 0 && which != 1 && which != 6 && which != 7) || n_seg < 0 || !total_zbytes ||
+    if (!c || (which != 0 && which != 1 && which != 6 && which != 7 && which != 9) || n_seg < 0 || !total_zbytes ||
         (n_seg > 0 && (!src_off || !nbytes || !file_off || !seg_zbytes)))
         return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
@@ -723,6 +724,18 @@ int ms_chain_write(ms_ctx* c, const int64_t* first_id, int64_t* chain_off) {
     if (!c || !first_id || !chain_off) return MS_ERR_ARG;
     MS_CUDA(c, cudaSetDevice(c->device));
     return chain_write(c, first_id, chain_off);
+}
+
+int ms_reads_size(ms_ctx* c, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count, int64_t* bytes) {
+    if (!c || !cfg || (c->n_contigs > 0 && (!n_pairs || !bytes))) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return reads_size(c, cfg, n_pairs, first, count, bytes);
+}
+
+int ms_reads_write(ms_ctx* c, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count, int64_t* nbytes) {
+    if (!c || !cfg || !nbytes || (c->n_contigs > 0 && !n_pairs)) return MS_ERR_ARG;
+    MS_CUDA(c, cudaSetDevice(c->device));
+    return reads_write(c, cfg, n_pairs, first, count, nbytes);
 }
 
 int ms_get_stats(ms_ctx* c, ms_stats* out) {

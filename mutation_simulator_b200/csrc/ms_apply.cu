@@ -1244,6 +1244,7 @@ int apply_pipeline(ms_ctx* c) {
     stage_end(c, ST_VCF);
     if ((rc = finish_apply(c))) return rc;
     c->chain_ready = true;
+    c->apply_full = true;
     return MS_OK;
 }
 

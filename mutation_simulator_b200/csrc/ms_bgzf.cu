@@ -159,8 +159,9 @@ __global__ void __launch_bounds__(THREADS) k_bgzf_pack(const uint8_t* __restrict
 int bgzf_compress(ms_ctx* c, int which, int32_t n_seg, const int64_t* src_off, const int64_t* nbytes, const int64_t* file_off,
                   const uint8_t* add_nl, int64_t* seg_zbytes, int64_t* total_zbytes) {
     const uint8_t* buf = which == 0 ? c->fasta.as<uint8_t>() : which == 1 ? c->vcf.as<uint8_t>()
-                       : which == 7 ? c->gt_vcf.as<uint8_t>() : c->chain.as<uint8_t>();
-    const int64_t size = which == 0 ? c->fasta_bytes : which == 1 ? c->vcf_bytes : which == 7 ? c->gt_vcf_bytes : c->chain_bytes;
+                       : which == 7 ? c->gt_vcf.as<uint8_t>() : which == 9 ? c->reads.as<uint8_t>() : c->chain.as<uint8_t>();
+    const int64_t size = which == 0 ? c->fasta_bytes : which == 1 ? c->vcf_bytes : which == 7 ? c->gt_vcf_bytes
+                       : which == 9 ? c->reads_bytes : c->chain_bytes;
     std::vector<Block> blocks;
     std::vector<int32_t> seg_of;
     for (int32_t s = 0; s < n_seg; ++s) {

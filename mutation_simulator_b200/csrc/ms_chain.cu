@@ -99,7 +99,8 @@ k_chain_down(ChainView v, int64_t n_items, const int64_t* __restrict__ tile_pref
 
 }  // namespace
 
-void chain_invalidate(ms_ctx* c) { c->chain_ready = false; c->chain_counted = false; c->chain_bytes = 0; }
+// (an apply output stops being current here, so the reads of a full apply go too)
+void chain_invalidate(ms_ctx* c) { c->chain_ready = false; c->chain_counted = false; c->chain_bytes = 0; reads_invalidate(c); }
 
 int chain_count(ms_ctx* c, int64_t* n_chains) {
     if (!c->chain_ready) MS_FAIL(c, MS_ERR_STATE, "ms_chain_count: no ms_apply / ms_apply_window output to describe");

@@ -9,6 +9,7 @@
 #include "ms_sample_core.h"
 #include "ms_tile_core.h"
 #include "ms_chain_core.h"
+#include "ms_reads_core.h"
 #include "../../include/mutsim_b200.h"
 
 namespace ms {
@@ -50,7 +51,8 @@ struct Totals {
 };
 
 enum Stage { ST_UPLOAD = 0, ST_SAMPLE_POS, ST_SAMPLE_TYPE, ST_SAMPLE_RESOLVE, ST_SAMPLE_LINK, ST_SAMPLE_FINAL,
-             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_CHAIN, ST_GENOTYPE, ST_SELECT, ST_VCF_PHASED, ST_COUNT };
+             ST_PLAN, ST_INDEX, ST_SPLICE, ST_VCF, ST_DOWNLOAD, ST_CHAIN, ST_GENOTYPE, ST_SELECT, ST_VCF_PHASED, ST_READS, ST_COUNT };
+static_assert(ST_COUNT <= (int)(sizeof(ms_stats::stage_ms) / sizeof(float)), "ms_stats.stage_ms has a slot per stage");
 
 }  // namespace ms
 
@@ -155,6 +157,16 @@ struct ms_ctx {
     int64_t gt_n_full = 0;        // records of the full table while a haplotype is selected
     bool gt_sizes_valid_full = false;
     int64_t gt_vcf_bytes = 0;
+
+    // paired-end reads (ms_reads.cu): FASTQ records of the last ms_reads_write (buffer 9), the per-pair draws and record
+    // offsets of the last sized range, the prefix of n_pairs, per-contig bytes
+    ms::DevBuf reads, reads_info, reads_off, reads_pre, reads_ctg;
+    int64_t reads_bytes = 0;
+    bool apply_full = false;      // buffer 0 and the active table's out positions describe the last full ms_apply
+    bool reads_sized = false;     // reads_info / reads_off hold the range below (ms_reads_size)
+    ms::ReadsCfg reads_cfg{};
+    int64_t reads_first = 0, reads_count = 0, reads_sized_total = 0;
+    std::vector<int64_t> h_reads_pre, reads_sized_pre;
 };
 
 #define MS_CUDA(ctx, call)                                                                        \
@@ -216,4 +228,7 @@ int genotype_draw(ms_ctx* c, uint64_t seed, int32_t ploidy, double hom_fraction)
 int genotype_load(ms_ctx* c, const uint8_t* masks, int64_t n, int32_t ploidy);
 int select_haplotype(ms_ctx* c, int32_t h);
 int vcf_phased(ms_ctx* c, int64_t* vcf_off);
+void reads_invalidate(ms_ctx* c);
+int reads_size(ms_ctx* c, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count, int64_t* bytes);
+int reads_write(ms_ctx* c, const ms_reads_cfg* cfg, const int64_t* n_pairs, int64_t first, int64_t count, int64_t* nbytes);
 }  // namespace ms

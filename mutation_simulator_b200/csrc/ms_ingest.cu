@@ -148,6 +148,7 @@ int fasta_ingest(ms_ctx* c, int fd, int32_t n_ranges, const int64_t* off, const 
     *n_records = 0; *regular = 0;
     c->fa_recs.clear(); c->fa_bytes = 0;
     c->fasta_bytes = 0; c->vcf_bytes = 0;      // the image takes over the FASTA output buffer: earlier outputs are gone
+    reads_invalidate(c);
     constexpr int64_t CH = ms_ctx::STAGE_BYTES;
     constexpr int NS = ms_ctx::N_STAGE;
     struct Chunk { int64_t foff, doff, n; };

@@ -68,6 +68,7 @@ enum Purpose : uint32_t {
     P_IT_KEY    = 7,   // the same for the breakpoint ranges of an interchromosomal pair (it_mutator.py:94-118)
     P_GENOME    = 8,   // synthetic genome generator (bench only)
     P_GENOTYPE  = 9,   // haplotype mask of one record of a polyploid run (ms_genotype_core.h)
+    P_READS     = 10,  // fragment, start, strand and errors of one read pair (ms_reads_core.h)
 };
 
 struct Seed { uint32_t k0, k1; };

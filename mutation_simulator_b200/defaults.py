@@ -23,6 +23,11 @@ class Defaults:
     # human sample (a documented default, not a measured claim)
     PLOIDY = 1
     HOM_FRACTION = 0.35
+    # --reads: a common short-read shape (2 x 150 bp, 500 bp inserts); documented choices, not measured claims
+    READ_LENGTH = 150
+    FRAGMENT_MEAN = 500
+    FRAGMENT_SD = 50
+    READ_ERROR_RATE = 0.001
 
 
 Defaults.MUT_BLOCK = {t: Defaults.BLOCK for t in (MutType.SN, MutType.IN, MutType.DE, MutType.IV, MutType.DU, MutType.TL, MutType.TLI)}

@@ -11,10 +11,10 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import MsRange, MsStats, MutSimError
+from ._lib import MsRange, MsReadsCfg, MsStats, MutSimError
 from .records import REC_DTYPE
 
-BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF, BUF_CHAIN, BUF_VCF_PHASED, BUF_GT = range(9)
+BUF_FASTA, BUF_VCF, BUF_RECS, BUF_LIT, BUF_GENOME, BUF_BGZF, BUF_CHAIN, BUF_VCF_PHASED, BUF_GT, BUF_READS = range(10)
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -340,7 +340,8 @@ class Engine:
         return int(nbytes)
 
     def bgzf_compress(self, which: int, src_off, nbytes, file_off, add_nl=None):
-        """BGZF members of segments of the FASTA image (which=0) or the VCF body (which=1), cut on 16 KiB cells of
+        """BGZF members of segments of the FASTA image (which=0), the VCF body (which=1), the chain text (6), the phased
+        VCF body (7) or the FASTQ records (9), cut on 16 KiB cells of
         the uncompressed file (ms_bgzf_compress); they become buffer BUF_BGZF.  Returns (compressed bytes of each
         segment, total)."""
         src_off, nbytes, file_off = (np.ascontiguousarray(a, dtype=np.int64) for a in (src_off, nbytes, file_off))
@@ -367,6 +368,29 @@ class Engine:
         self._check(self._lib.ms_chain_write(self._h, _ptr(first), _ptr(off)))
         self.chain_off = off
         return off
+
+    @staticmethod
+    def _reads_cfg(cfg: dict) -> MsReadsCfg:
+        return MsReadsCfg(C.c_uint64(int(cfg["seed"]) & 0xFFFFFFFFFFFFFFFF).value, int(cfg["hap"]), int(cfg["read_len"]),
+                          int(cfg["frag_mean"]), int(cfg["frag_sd"]), float(cfg["error_rate"]), int(cfg["qual"]))
+
+    def reads_size(self, cfg: dict, n_pairs, first: int, count: int) -> np.ndarray:
+        """Bytes one FASTQ file's records of pairs [first, first + count) take in each contig (ms_reads_size).  cfg: seed,
+        hap, read_len, frag_mean, frag_sd, error_rate, qual; n_pairs: pairs of each contig, numbered contig-major."""
+        n = np.ascontiguousarray(n_pairs, dtype=np.int64)
+        out = np.zeros(self.n_contigs, dtype=np.int64)
+        c = self._reads_cfg(cfg)
+        self._check(self._lib.ms_reads_size(self._h, C.byref(c), _ptr(n), int(first), int(count), _ptr(out)))
+        return out
+
+    def reads_write(self, cfg: dict, n_pairs, first: int, count: int) -> int:
+        """Format pairs [first, first + count) into buffer BUF_READS: R1 records at [0, n), R2 records at [n, 2n)
+        (ms_reads_write).  Returns n."""
+        n = np.ascontiguousarray(n_pairs, dtype=np.int64)
+        nb = C.c_int64()
+        c = self._reads_cfg(cfg)
+        self._check(self._lib.ms_reads_write(self._h, C.byref(c), _ptr(n), int(first), int(count), C.byref(nb)))
+        return nb.value
 
     def fasta(self) -> bytes:
         return self.download(BUF_FASTA).tobytes()

@@ -7,7 +7,10 @@ Nothing here touches a base on the host.
 
 With ``--ploidy P`` >= 2 the same table is sampled, every record draws its haplotype mask on the GPU, the phased VCF of
 the whole table is written, and then each haplotype's records are selected on the device and applied in turn: one
-FASTA (and chain) per haplotype."""
+FASTA (and chain) per haplotype.
+
+With ``--reads`` each haplotype's read pairs are drawn right after its FASTA (and chain) is written, while its mutated
+genome is still in HBM, and appended to ``*_ms_R1.fq`` / ``*_ms_R2.fq`` (reads_writer.py)."""
 from __future__ import annotations
 
 import os
@@ -32,7 +35,8 @@ def run_seed(args) -> int:
 
 
 class Mutator:
-    def __init__(self, args, fasta, sim):
+    def __init__(self, args, fasta, sim, reads_budget=None):
+        """reads_budget: FASTQ bytes formatted in HBM per call with --reads (default reads_writer.DEFAULT_BATCH_BYTES)."""
         self._args, self._fasta, self._sim = args, fasta, sim
         self._rank, self._world = D.init()
         self._engine = None
@@ -40,9 +44,17 @@ class Mutator:
         self._replay = None
         self._ploidy = getattr(args, "ploidy", 1)
         self._hap_writers = []
+        self._reads_writer = None
+        self._reads_pairs = None         # pairs per contig over the haplotypes written so far (for the empty-contig warning)
+        from .reads_writer import DEFAULT_BATCH_BYTES
+        self._reads_budget = reads_budget or DEFAULT_BATCH_BYTES
         # plan the ranges (and reject overlapping ones) BEFORE any output file is opened and truncated: a settings
         # error must not leave partial *_ms.fa / *_ms.vcf behind (the reference dies later, with both files cut)
         self._planned = build_ranges(sim, fasta.lengths, None) if sim.has_mutations else None
+        if getattr(args, "reads", None) is not None:
+            from .reads_writer import ReadsWriter
+            self._reads_writer = ReadsWriter([args.outreads1, args.outreads2], getattr(args, "bgzip", False), self._reads_budget,
+                                             create=self._world == 1)
         if self._world > 1:      # one process per GPU: files are assembled by write_partitioned()
             self._fasta_writer = self._vcf_writer = None
             return
@@ -74,6 +86,9 @@ class Mutator:
     def close(self):
         for w in self._hap_writers:
             w.close()
+        if self._reads_writer is not None:
+            self._reads_writer.close()
+            self._reads_writer = None
         if self._fasta_writer is not None:
             self._fasta_writer.close()
         if self._vcf_writer is not None:
@@ -102,7 +117,7 @@ class Mutator:
         my_ids = D.partition_of(fasta, world)[self._rank] if world > 1 and not tiles else list(range(n_contigs))
         self.shard, self.my_ids = ("tiles" if tiles else "contigs"), my_ids
         self.parts = D.partition_of(fasta, world) if world > 1 and not tiles else None
-        seed = D.broadcast_object(run_seed(args))
+        seed = self._seed = D.broadcast_object(run_seed(args))
         eng = self._engine = getattr(fasta, "engine", None) or \
             Engine(D.local_device(getattr(args, "device", 0)) if world > 1 else getattr(args, "device", 0))
         lap("engine")
@@ -180,6 +195,10 @@ class Mutator:
             if chain:
                 self._write_chain_partitioned(eng, tiles, my_ids, n_contigs, bgzip)
         lap("download+write")
+        if self._reads_writer is not None:
+            self._write_reads(eng, 1, tiles, my_ids, n_contigs)
+            self._warn_no_reads(tiles, my_ids)
+            lap("reads")
         self._finish(eng, my_ids, marks)
 
     def _finish(self, eng, my_ids, marks):
@@ -237,10 +256,42 @@ class Mutator:
                     write_from_engine(args.outchains[h - 1], eng, bgzip)
                 else:
                     self._write_chain_partitioned(eng, tiles, my_ids, n_contigs, bgzip, args.outchains[h - 1])
+            if self._reads_writer is not None:
+                self._write_reads(eng, h, tiles, my_ids, n_contigs)
         lap("haplotypes")
+        if self._reads_writer is not None:
+            self._warn_no_reads(tiles, my_ids)
         if my_ids and not args.ignore_warnings and (not tiles or self._rank == 0) and getattr(args, "mode", None) != "vcf":
             self._warn_empty(per, my_ids)        # a contig that no haplotype mutates got no records at all
         self._finish(eng, my_ids, marks)
+
+    def _write_reads(self, eng, h, tiles, my_ids, n_contigs):
+        """Haplotype h's read pairs from the mutated genome of its apply, appended to both FASTQ files.  Tile mode: every
+        rank applies the whole haplotype (the window apply leaves buffer 0 partly valid) and writes pairs
+        [n r / W, n (r + 1) / W) of each contig; contig mode: each rank writes its contigs' pairs."""
+        from .reads_writer import config, pair_counts
+        args, world, rank = self._args, self._world, self._rank
+        cfg = config(args, self._seed, h)
+        n = np.zeros(len(my_ids), dtype=np.int64)
+        if my_ids:
+            if tiles:
+                eng.apply()
+            n = pair_counts(args.reads, eng.contig_out_len(), args.read_length, self._ploidy)
+        self._reads_pairs = n if self._reads_pairs is None else self._reads_pairs + n
+        if world == 1:
+            self._reads_writer.write(eng, cfg, n)
+        elif tiles:
+            slices = [(g * world + rank, g, int(n[g]) * rank // world, int(n[g]) * (rank + 1) // world) for g in range(len(my_ids))]
+            self._reads_writer.write_partitioned(eng, cfg, n, slices, n_contigs * world)
+        else:
+            self._reads_writer.write_partitioned(eng, cfg, n, [(g, i, 0, int(n[i])) for i, g in enumerate(my_ids)], n_contigs)
+
+    def _warn_no_reads(self, tiles, my_ids):
+        if not my_ids or self._args.ignore_warnings or (tiles and self._rank != 0):
+            return
+        for i in np.flatnonzero(self._reads_pairs == 0):
+            print(format_warning(f"No reads could be simulated on sequence {my_ids[int(i)]+1} (shorter than the read length or "
+                                 "depth too low)", self._args.no_color), file=sys.stderr)
 
     def _warn_empty(self, per_contig, my_ids):
         for i in np.flatnonzero(per_contig == 0):
